@@ -2,6 +2,7 @@
 """Benchmark of the ProxyTTA per-frame adaptation step (BASELINE.json: adapted frames/s, fwd+bwd+update, 352x1216).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload kitti|void|nlspn|prepare_init|prepare_head|prepare_head_nlspn] [--batch B]
+                    [--dump-outputs DIR]
 
 One "step" = src/tta_main.py:583-633 of the reference for one batch: outlier removal, forward (real + zero-image
 branch + proxy heads), the three losses, backward to the adapted meta layer, Adam.  Workload at N=1 = BASELINE.json
@@ -15,7 +16,11 @@ facade with HOST pinned inputs, H2D inside the timed region, loss read back D2H 
 
 `--impl reference`: the reference's own CPU path -- here the oracle port of it (the reference is PyTorch-eager Python
 that cannot travel to the GPU box; oracle/msgchn_oracle.py is pinned against its outputs, tests/golden/) -- timed on
-all host cores on the same workload."""
+all host cores on the same workload.
+
+`--dump-outputs DIR`: after the timed steps, what the last timed step handed its caller (output depth where the step makes one,
+loss values, adapted or trained parameters) is written to DIR/<name>.npy.  Inputs and starting weights are seeded, so two builds
+run with the same arguments can be compared file by file."""
 import argparse
 import json
 import os
@@ -170,6 +175,28 @@ def make_checkpoint(workload):
     return synthetic.make_synthetic_checkpoint(0, WORKLOADS[workload][3])
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+NPY_HEADER_BYTES = 128          # what np.save writes in front of a 1-D or small-rank float array
+
+
+def dump_outputs(out_dir, arrays):
+    """`--dump-outputs`: {name: CPU tensor or Python float} -> out_dir/<name>.npy (tensors as float32, scalars as float64), at most
+    DUMP_LIMIT_BYTES of files in all.  Arrays are written smallest first; one that does not fit in what the smaller ones left, split
+    evenly over it and the larger ones, is replaced by a fixed sample of its flattened values (indices drawn with seed 0, kept in
+    ascending order), so that runs with the same arguments write the same elements."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: (v.float().numpy() if isinstance(v, torch.Tensor) else np.float64(v)) for k, v in arrays.items()}
+    left = DUMP_LIMIT_BYTES
+    for i, (name, a) in enumerate(sorted(arrays.items(), key=lambda kv: kv[1].nbytes)):
+        share = left // (len(arrays) - i) - NPY_HEADER_BYTES
+        if a.nbytes > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False))]
+        path = os.path.join(out_dir, name + '.npy')
+        np.save(path, a)
+        left -= os.path.getsize(path)
+
+
 # ------------------------------------------------------------------------------------------------------------
 def nlspn_cpu_sample(args, steps, warmup):
     """NLSPN oracle port on the host cores.  A full 352x1216 step needs ~25 GB of fp32 activations and minutes on CPU, so the
@@ -255,7 +282,7 @@ def run_reference(args):
     if rank != 0:
         return
     if args.workload in PREPARE:
-        steps, warm = min(args.steps, 5), min(args.warmup, 1)
+        steps, warm = args.steps, min(args.warmup, 1)
         dt = prepare_cpu_steps(args, steps, warm)
         value = args.batch / dt
         h, w = WORKLOADS[args.workload][:2]
@@ -268,7 +295,7 @@ def run_reference(args):
                           'e2e': {'value': value, 'unit': 'frames/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0}}), flush=True)
         return
     if args.workload.startswith('nlspn'):
-        steps = min(args.steps, 3)
+        steps = args.steps
         value, dt, cb = nlspn_cpu_sample(args, steps, min(args.warmup, 1))
         print(json.dumps({'impl': 'reference', 'metric': 'adapted_frames_per_sec', 'value': value, 'unit': 'frames/s', 'n_gpus': args.gpus,
                           'steps': steps, 'warmup': min(args.warmup, 1), 'ms_per_step': 1e3 * 4.0 * dt / steps, 'higher_is_better': True,
@@ -505,6 +532,9 @@ def run_native_nlspn(args):
         ms_total = e0.elapsed_time(e1)
         sampler.stop_flag = True
         losses = eng.read_losses()
+        if args.dump_outputs and rank == 0:             # taken before the e2e leg adapts the model further
+            dumped = dict(losses, output_depth=eng.B['output'].cpu(),
+                          adapted_parameters=torch.cat([eng.params[k].reshape(-1) for k in eng.adapt_names]).cpu())
         pre = HostPrefetcher(pinned, img_d, sp_d, stream, dev)
         pre.consumed[0].record(stream); pre.consumed[1].record(stream)
         pre.prefetch(0)
@@ -550,6 +580,8 @@ def run_native_nlspn(args):
         line['roofline'] = time_convg_kernel(dev, peaks)
         line['cpu_baseline'] = nlspn_cpu_sample(args, 1, 1)[2]
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 
@@ -746,6 +778,13 @@ def run_native_prepare(args):
         ms_total = e0.elapsed_time(e1)
         sampler.stop_flag = True
         losses = model.last_losses()
+        if args.dump_outputs and rank == 0:             # taken before the e2e passes train further
+            from tta_depth_completion_b200.nlspn_prepare import HEAD_TRAINED
+            sd = model.state_dict()
+            trained = HEAD_TRAINED if nlspn else model.model._adapt_names
+            dumped = dict(losses, trained_parameters=torch.cat([sd[k].reshape(-1) for k in trained]).cpu())
+            if stage == 'init':
+                dumped['output_depth'] = model.last_output().cpu()
         # end to end: pinned host frames -> H2D -> step -> D2H loss read (synchronising), every step
         passes = []
         for _ in range(E2E_PASSES):
@@ -788,6 +827,8 @@ def run_native_prepare(args):
                                 'sample': '2 full-size %s steps (%dx3x%dx%d) of oracle/%s_oracle.py (torch %s CPU fp32) after 1 warm-up, %.2f s/step' % (
                                     stage, args.batch, h, w, 'nlspn' if nlspn else 'msgchn', torch.__version__, dt)}
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 
@@ -875,6 +916,9 @@ def run_native(args):
         ms_total = e0.elapsed_time(e1)
         sampler.stop_flag = True
         losses = model.last_losses()
+        if args.dump_outputs and rank == 0:             # taken before the e2e and drop-in legs adapt the model further
+            dumped = dict(losses, output_depth=model.last_output().cpu(),
+                          adapted_parameters=torch.cat([p.detach().reshape(-1) for p in model.adapt_parameters('meta')]).cpu())
 
         # ---- end to end: host pinned inputs -> H2D -> step -> D2H loss read, every step -------------------------------
         # E2E_PASSES passes of `steps` steps each, every pass bracketed like the device-resident region; the MEDIAN pass is reported
@@ -957,6 +1001,8 @@ def run_native(args):
         line['gpu_eager_baseline'] = gpu_eager_baseline(args, dev)
         line['cpu_baseline'] = cpu_baseline_sample(args)
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 
@@ -974,10 +1020,18 @@ def main():
     ap.add_argument('--inner-iter', type=int, default=1, help='adaptation steps per frame (src/tta_main.py:579; the indoor script bash/adapt/adapt_msgchn_scenenet.sh runs 3); a bench "step" is then one FRAME = inner_iter TTA steps')
     ap.add_argument('--no-extras', action='store_true', help='skip the roofline / cpu_baseline legs (profiling runs)')
     ap.add_argument('--engine-opt', action='append', default=[], metavar='NAME=VALUE', help='ptta_msgchn_set_option on the engine (dispatch experiments, e.g. tc_min_pixels=1000); not for headline runs')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step computed to DIR/<name>.npy (float32 / float64, at most 64 MB in all)')
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.steps is None:
-        args.steps = 10 if args.impl == 'reference' else 200
+        if args.impl == 'reference':          # a CPU step of these workloads takes seconds to minutes
+            args.steps = 5 if args.workload in PREPARE else 3 if args.workload.startswith('nlspn') else 10
+        else:
+            args.steps = 200
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs records the native path (--impl native)')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -2,10 +2,14 @@
 restoring its 'net' + torch.optim.Adam state into the oracle and taking the next step reproduces what the reference did next."""
 import os
 
+import pytest
 import torch
 
 from golden_util import GOLDEN_DIR, load_golden, case_frame, rel, nrel, W_SD, W_SM, W_COS
+from golden_util import fixture_threads  # noqa: F401  (pytest fixture)
 from oracle import msgchn_oracle as O
+
+pytestmark = pytest.mark.usefixtures('fixture_threads')
 
 NAME = 'refckpt_2layers_kitti_1x64x128'
 

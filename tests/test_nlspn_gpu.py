@@ -1,7 +1,7 @@
 """GPU tier: the B200 NLSPN propagation kernels (through the C ABI / nlspn_prop.py) against the oracle, the fixtures generated
-by the reference's own NLSPN class, and -- when oracle/_ref/dcn_ref.so travelled with the snapshot -- the reference's own DCN
-CUDA kernels.  Tolerances: fp32 arithmetic in a different summation order -> 1e-5 relative (norm-wise) on values and
-gradients; scatter-accumulated gradients (fp32 atomics, as in the reference) 1e-4."""
+by the reference's own NLSPN class, torchvision's DCNv2, and -- where oracle/build_ref_dcn.py has built oracle/_ref/dcn_ref.so
+from the reference's source -- the reference's own DCN CUDA kernels.  Tolerances: fp32 arithmetic in a different summation order
+-> 1e-5 relative (norm-wise) on values and gradients; scatter-accumulated gradients (fp32 atomics, as in the reference) 1e-4."""
 import importlib.machinery
 import importlib.util
 import os
@@ -69,18 +69,35 @@ def test_mdconv_matches_oracle(NP, n, h, w, k, pad):
         assert rel(got, torch.from_numpy(np.ascontiguousarray(ref_))) < tol, name
 
 
+def reference_mdconv(impl, x, off, m, wt, b, go, k, pad):
+    """(output, [grad_input, grad_offset, grad_mask, grad_weight, grad_bias]) of a reference DCNv2 on CPU tensors:
+    'reference_kernels': the reference's own CUDA kernels (oracle/_ref/dcn_ref.so);
+    'torchvision': torchvision's deform_conv2d with a mask (the reference's offset layout and bilinear border rule) on the CPU,
+    in float32 as the reference -- a sampling position rounded differently can land in the neighbouring cell, where the offset
+    gradient jumps (in float64, about 1e-2 of it moves at 352x1216)."""
+    if impl == 'reference_kernels':
+        ref = dcn_ref()
+        if ref is None:
+            pytest.skip('oracle/_ref/dcn_ref.so not built (oracle/build_ref_dcn.py builds it from the reference\'s source tree)')
+        x, off, m, wt, b, go = (t.to(DEV) for t in (x, off, m, wt, b, go))
+        want = ref.modulated_deform_conv_forward(x, wt, b, off, m, k, k, 1, 1, pad, pad, 1, 1, 1, 1, 64)
+        return want, ref.modulated_deform_conv_backward(x, wt, b, off, m, go, k, k, 1, 1, pad, pad, 1, 1, 1, 1, 64)
+    tvops = pytest.importorskip('torchvision.ops')
+    cpu = [t.clone().requires_grad_(True) for t in (x, off, m, wt, b)]
+    want = tvops.deform_conv2d(cpu[0], cpu[1], cpu[3], cpu[4], stride=1, padding=pad, dilation=1, mask=cpu[2])
+    want.backward(go)
+    return want, [t.grad for t in cpu]
+
+
 @pytest.mark.parametrize('n,h,w,k,pad', [(2, 40, 72, 3, 1), (1, 40, 72, 1, 0), (1, 352, 1216, 3, 1)])
-def test_mdconv_matches_the_references_cuda_kernels(NP, n, h, w, k, pad):
-    ref = dcn_ref()
-    if ref is None:
-        pytest.skip('oracle/_ref/dcn_ref.so not built (python oracle/build_ref_dcn.py where /root/reference is mounted)')
-    x, off, m, wt, b, go = (t.to(DEV) for t in rand_case(4, n, h, w, k))
-    want = ref.modulated_deform_conv_forward(x, wt, b, off, m, k, k, 1, 1, pad, pad, 1, 1, 1, 1, 64)
-    gwant = ref.modulated_deform_conv_backward(x, wt, b, off, m, go, k, k, 1, 1, pad, pad, 1, 1, 1, 1, 64)
-    dx, doff, dm, dw, db = (t.clone().requires_grad_(True) for t in (x, off, m, wt, b))
+@pytest.mark.parametrize('impl', ['reference_kernels', 'torchvision'])
+def test_mdconv_matches_reference_dcn(NP, impl, n, h, w, k, pad):
+    x, off, m, wt, b, go = rand_case(4, n, h, w, k)
+    want, gwant = reference_mdconv(impl, x, off, m, wt, b, go, k, pad)
+    dx, doff, dm, dw, db = (t.to(DEV).requires_grad_(True) for t in (x, off, m, wt, b))
     out = NP.ModulatedDeformConvFunction.apply(dx, doff, dm, dw, db, 1, pad, 1, 1, 1, 64)
     assert rel(out, want) < 1e-5
-    out.backward(go)
+    out.backward(go.to(DEV))
     for got, ref_, name, tol in ((dx.grad, gwant[0], 'grad_input', 1e-4), (doff.grad, gwant[1], 'grad_offset', 1e-5),
                                  (dm.grad, gwant[2], 'grad_mask', 1e-5), (dw.grad, gwant[3], 'grad_weight', 1e-3), (db.grad, gwant[4], 'grad_bias', 1e-3)):
         assert rel(got, ref_) < tol, (name, rel(got, ref_))

@@ -6,7 +6,9 @@ import torch
 
 from oracle import msgchn_oracle as O
 from golden_util import golden_names, load_golden, case_frame, case_checkpoint, rel, nrel, W_SD, W_SM, W_COS
+from golden_util import fixture_threads  # noqa: F401  (pytest fixture)
 
+pytestmark = pytest.mark.usefixtures('fixture_threads')
 # fp32 CPU vs fp32 CPU of the same torch build: only summation-order noise is expected
 TOL_LOSS = 2e-5
 TOL_TENSOR = 2e-5

@@ -9,7 +9,10 @@ import torch
 
 from oracle import msgchn_oracle as O
 from golden_util import GOLDEN_DIR, nrel, rel
+from golden_util import fixture_threads  # noqa: F401  (pytest fixture)
 from tta_depth_completion_b200.external_model_adapt import add_head_state
+
+pytestmark = pytest.mark.usefixtures('fixture_threads')
 
 # a bias in front of a train-mode BatchNorm has an analytically zero gradient: both sides hold rounding noise there and Adam turns its
 # SIGN into +-lr steps, so these tensors are only bounded by the distance Adam can move them

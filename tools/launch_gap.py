@@ -1,5 +1,5 @@
 import sys, os, torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from tta_depth_completion_b200 import _lib
 from tta_depth_completion_b200._lib import ptr, c_void_p
 L = _lib.lib()
