@@ -23,6 +23,7 @@ extern "C" {
 
 typedef void* ptta_stream_t;            /* cudaStream_t */
 typedef struct ptta_msgchn ptta_msgchn; /* opaque engine */
+typedef struct ptta_comm ptta_comm;     /* peer communicator of the shared-model mode (below) */
 
 const char* ptta_last_error(void);
 int ptta_version(void);
@@ -121,6 +122,11 @@ int ptta_adam_flat(float* param, const float* grad, float* exp_avg, float* exp_a
  * (doubles) in DEVICE memory, so the call can be captured into a CUDA graph and replayed */
 int ptta_adam_flat_dev(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, const double* hyper_dev,
                        int* step_dev, ptta_stream_t stream);
+/* shared-model mode of the same update (ptta_comm, below): the flat gradient buffer is mean-all-reduced over the ranks inside the kernel
+ * (ranks summed in rank order, bit-identical on all of them), the average is written back to grad, then the update runs.  xid: the
+ * exchange id of the call within the step (all ranks issue the same sequence).  n <= the communicator's grad_floats. */
+int ptta_adam_flat_dev_comm(float* param, float* grad, float* exp_avg, float* exp_avg_sq, long long n, const double* hyper_dev,
+                            int* step_dev, ptta_comm* comm, int xid, ptta_stream_t stream);
 
 /* ---- NLSPN non-local spatial propagation (SURVEY.md section 8 a20-a21) ----------------------------- */
 /* DCN.modulated_deform_conv_forward / _backward, the reference's one native FFI
@@ -257,6 +263,17 @@ int ptta_nl_bn_backward(const void* dy_a, long long ld_a, const void* dy_b, long
                         const void* x_bf16, const float* mean, const float* rstd, const float* gamma, float* partial,
                         float* dgamma, float* dbeta, float* coef, void* dx_bf16, void* gskip_bf16, long long rows, int c,
                         ptta_stream_t stream);
+/* shared-model mode (SyncBatchNorm over the ranks of `comm`): the same two calls with the per-channel sums exchanged through peer memory
+ * inside the finalize kernel and added in rank order; count = rows x world.  xid: the exchange id of the call within the step.  The
+ * backward's dgamma / dbeta stay the LOCAL sums (the gradient all-reduce averages them, as DDP does); dx uses the global means.  c <= 1024.
+ * Every rank must issue the same sequence of exchanges, on one stream. */
+int ptta_nl_bn_stats_comm(const void* x_bf16, long long ldx, long long rows, int c, const float* gamma, const float* beta, float eps,
+                          float* partial, float* mean, float* rstd, float* scale, float* shift, float* run_mean, float* run_var,
+                          long long* num_batches_tracked, float momentum, ptta_comm* comm, int xid, ptta_stream_t stream);
+int ptta_nl_bn_backward_comm(const void* dy_a, long long ld_a, const void* dy_b, long long ld_b, const void* y_bf16, int act,
+                             const void* x_bf16, const float* mean, const float* rstd, const float* gamma, float* partial,
+                             float* dgamma, float* dbeta, float* coef, void* dx_bf16, void* gskip_bf16, long long rows, int c,
+                             ptta_comm* comm, int xid, ptta_stream_t stream);
 int ptta_nl_add3(const void* a, long long lda, const void* b, long long ldb, const void* c3, long long ldc, void* out, long long rows,
                  int c, ptta_stream_t stream);
 /* output = clamp(y, min=0) (nlspnmodel_adapt.py:901) and its adjoint */
@@ -363,13 +380,17 @@ void ptta_msgchn_destroy(ptta_msgchn* e);
  * summed in rank order: bit-identical replicas).  No NCCL call on the path; the step stays capturable in one CUDA graph.
  * Train-mode BatchNorm sums: exchanged inside bn_finalize / bn_bwd_finalize.  Host protocol: create -> local_handle -> exchange the handles (any transport, e.g. torch.distributed.all_gather_object) ->
  * open_peers -> ptta_msgchn_set_comm. */
-typedef struct ptta_comm ptta_comm;
 int ptta_comm_create(ptta_comm** out, int rank, int world, long long grad_floats);
 int ptta_comm_handle_bytes(void);
 int ptta_comm_local_handle(ptta_comm* c, void* handle_out);
 int ptta_comm_open_peers(ptta_comm* c, const void* handles_world_x_bytes);
 int ptta_comm_error(ptta_comm* c);      /* 0 = fine; k > 0 = exchange k-1 timed out waiting for a peer (~4 s): results are void */
 void ptta_comm_destroy(ptta_comm* c);
+/* exchanges one step may use (exchange ids 0 .. max-1) */
+int ptta_comm_max_exchanges(void);
+/* end of a step driven through the ptta_*_comm entry points: the next step's exchanges use the next tag (the MSG-CHN engine does this
+ * inside its Adam step) */
+int ptta_comm_advance(ptta_comm* c, ptta_stream_t stream);
 int ptta_msgchn_set_comm(ptta_msgchn* e, ptta_comm* c);
 int ptta_msgchn_set_option(ptta_msgchn* e, const char* name, long long value);
 size_t ptta_msgchn_workspace_bytes(const ptta_msgchn* e);

@@ -1773,6 +1773,39 @@ __global__ void adam_flat_dev_kernel(float* p, const float* g, float* m, float* 
         p[i] = pp; m[i] = mm; v[i] = vv;
     }
 }
+// shared-model mode of the flat-buffer Adam (the NLSPN back-end): mean all-reduce of the gradient buffer FUSED with the update, one-shot
+// over peer memory like adam_allreduce_kernel.  Block = one ADAM_CHUNK slice of the buffer: it copies its slice of the local gradient into
+// the rank's slot, the ranks rendezvous (peer_comm.cuh), then it sums the W copies in rank order (bit-identical on all ranks), scales by
+// 1/W, writes the averaged gradient back to g (what DDP leaves in .grad) and applies the update of adam_flat_dev_kernel
+__global__ void __launch_bounds__(256) adam_flat_allreduce_kernel(float* __restrict__ p, float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                                                                  long long n, const double* __restrict__ hy, const int* __restrict__ step,
+                                                                  const PeerComm comm, int xid) {
+    PDL_SYNC();
+    const long long i0 = (long long)blockIdx.x * ADAM_CHUNK;
+    const int cnt = n - i0 < ADAM_CHUNK ? (int)(n - i0) : ADAM_CHUNK;
+    const uint32_t tag = comm_tag(comm);
+    const size_t off = comm_grad_off((int)(tag & 1u), comm.grad_floats);
+    float* mine = reinterpret_cast<float*>(comm.base[comm.rank] + off) + i0;
+    for (int i = threadIdx.x; i < cnt; i += 256) mine[i] = g[i0 + i];
+    comm_publish_and_wait(comm, xid, tag);
+    const double b1 = hy[1], b2 = hy[2];
+    const int t = *step;
+    const double bc1 = 1.0 - pow(b1, (double)t);
+    const double bc2 = 1.0 - pow(b2, (double)t);
+    const float step_size = (float)(hy[0] / bc1);
+    const float bc2_sqrt = (float)sqrt(bc2);
+    const float fb2 = (float)b2, omb1 = (float)(1.0 - b1), omb2 = (float)(1.0 - b2), eps = (float)hy[3], wd = (float)hy[4];
+    const float inv_w = 1.f / (float)comm.world;
+    for (int i = threadIdx.x; i < cnt; i += 256) {
+        float gs = 0.f;
+        for (int r = 0; r < comm.world; ++r) gs += ld_volatile_f32(reinterpret_cast<const float*>(comm.base[r] + off) + i0 + i);
+        gs *= inv_w;
+        g[i0 + i] = gs;
+        float pp = p[i0 + i], mm = m[i0 + i], vv = v[i0 + i];
+        adam_update(pp, gs, mm, vv, fb2, omb1, omb2, eps, wd, step_size, bc2_sqrt);
+        p[i0 + i] = pp; m[i0 + i] = mm; v[i0 + i] = vv;
+    }
+}
 // ---- stand-alone fused TTA loss (used by the NLSPN back-end, whose graph is driven from Python) -------------------------------------
 struct TtaLossLayout { size_t scalars, map_partial, cos_partial, rowstat, total; int map_blocks, cos_blocks; };
 static TtaLossLayout tta_loss_layout(int n, int h, int w, long long rows) {
@@ -1992,6 +2025,24 @@ int ptta_adam_flat_dev(float* p, const float* g, float* m, float* v, long long n
     return check_launch("adam_flat_dev");
 }
 
+int ptta_adam_flat_dev_comm(float* p, float* g, float* m, float* v, long long n, const double* hyper_dev, int* step_dev, ptta_comm* comm, int xid,
+                            ptta_stream_t stream) {
+    PTTA_CHECK(p && g && m && v && hyper_dev && step_dev && comm, "adam_flat_dev_comm: null pointer");
+    PTTA_CHECK(xid >= 0 && xid < PTTA_COMM_MAX_XID, "adam_flat_dev_comm: exchange id %d outside [0, %d)", xid, PTTA_COMM_MAX_XID);
+    PTTA_CHECK(n > 0 && (size_t)n <= comm->dev.grad_floats, "adam_flat_dev_comm: %lld floats, the communicator's gradient slot holds %zu", n,
+               comm->dev.grad_floats);
+    // every block spins in the rendezvous: all of them must be resident at once (peer_comm.cuh: a spinning kernel has at most
+    // PTTA_COMM_MAX_SPIN_BLOCKS blocks; the NLSPN buffer needs 23)
+    const long long blocks = cdiv(n, (long long)ADAM_CHUNK);
+    PTTA_CHECK(blocks <= PTTA_COMM_MAX_SPIN_BLOCKS, "adam_flat_dev_comm: %lld floats need %lld blocks (at most %d spin at once)", n, blocks,
+               PTTA_COMM_MAX_SPIN_BLOCKS);
+    for (int r = 0; r < comm->dev.world; ++r) PTTA_CHECK(comm->dev.base[r] != nullptr, "adam_flat_dev_comm: peer %d not opened (ptta_comm_open_peers)", r);
+    launch_k(adam_tick_kernel, 1, 1, 0, (cudaStream_t)stream, step_dev);
+    PTTA_TRY(check_launch("adam_tick"));
+    launch_k(adam_flat_allreduce_kernel, (int)blocks, 256, 0, (cudaStream_t)stream, p, g, m, v, n, hyper_dev, step_dev, comm->dev, xid);
+    return check_launch("adam_flat_allreduce");
+}
+
 // ---- NLSPN propagation path (SURVEY.md section 8 a20-a21) ------------------------------------------------------
 static int mdconv_check(int c_in, int c_out, int kh, int kw, int stride, int pad, int dil, int groups, int dgroups) {
     PTTA_CHECK(c_in == 1 && c_out == 1 && groups == 1 && dgroups == 1,
@@ -2125,12 +2176,7 @@ int ptta_msgchn_create(ptta_msgchn** out, int n, int h, int w, const char* prepa
     return 0;
 }
 // ---- peer communicator of the shared-model mode (peer_comm.cuh) ---------------------------------------------------------
-struct ptta_comm {
-    PeerComm dev;
-    void* local = nullptr;
-    void* opened[PTTA_COMM_MAX_RANKS] = {};
-    size_t bytes = 0;
-};
+// struct ptta_comm: peer_comm.cuh (the NLSPN entry points of nlspn_net.cu read its device view too)
 int ptta_comm_create(ptta_comm** out, int rank, int world, long long grad_floats) {
     PTTA_CHECK(out && world >= 1 && world <= PTTA_COMM_MAX_RANKS && rank >= 0 && rank < world && grad_floats > 0, "comm_create: bad arguments (rank %d of %d)", rank, world);
     ptta_comm* c = new ptta_comm();
@@ -2178,6 +2224,12 @@ void ptta_comm_destroy(ptta_comm* c) {
     for (int r = 0; r < PTTA_COMM_MAX_RANKS; ++r) if (c->opened[r]) cudaIpcCloseMemHandle(c->opened[r]);
     if (c->local) cudaFree(c->local);
     delete c;
+}
+int ptta_comm_max_exchanges(void) { return PTTA_COMM_MAX_XID; }
+int ptta_comm_advance(ptta_comm* c, ptta_stream_t stream) {
+    PTTA_CHECK(c && c->local, "comm_advance: null communicator");
+    launch_k(comm_advance_kernel, 1, 32, 0, (cudaStream_t)stream, c->dev);
+    return check_launch("comm_advance");
 }
 /* shared-model mode on: SyncBatchNorm statistics over all ranks + gradient all-reduce fused with Adam (comm = NULL: off).  Exchange slots
  * are numbered in host call order, which is the same on every rank; kernels of different streams may reach their exchanges in any

@@ -184,6 +184,49 @@ int ptta_nl_bn_backward(const void* dy_a, long long ld_a, const void* dy_b, long
     return check_launch("nl_bn_bwd_apply");
 }
 
+// shared-model mode: the communicator must have every peer mapped, and one BatchNorm's sums must fit an exchange slot
+static int comm_check(const ptta_comm* comm, int xid, int c, const char* what) {
+    PTTA_CHECK(comm, "%s: null communicator", what);
+    PTTA_CHECK(xid >= 0 && xid < PTTA_COMM_MAX_XID, "%s: exchange id %d outside [0, %d)", what, xid, PTTA_COMM_MAX_XID);
+    PTTA_CHECK(2 * c <= PTTA_COMM_BN_DOUBLES, "%s: %d channels exceed the exchange slot (%d)", what, c, PTTA_COMM_BN_DOUBLES / 2);
+    for (int r = 0; r < comm->dev.world; ++r) PTTA_CHECK(comm->dev.base[r] != nullptr, "%s: peer %d not opened (ptta_comm_open_peers)", what, r);
+    return 0;
+}
+
+int ptta_nl_bn_stats_comm(const void* x, long long ldx, long long rows, int c, const float* gamma, const float* beta, float eps, float* partial,
+                          float* mean, float* rstd, float* scale, float* shift, float* run_mean, float* run_var, long long* num_batches_tracked,
+                          float momentum, ptta_comm* comm, int xid, ptta_stream_t stream) {
+    PTTA_CHECK(x && gamma && beta && partial && mean && rstd && scale && shift && c % 64 == 0 && rows > 0, "nl_bn_stats_comm: bad arguments");
+    PTTA_TRY(comm_check(comm, xid, c, "nl_bn_stats_comm"));
+    const int nblk = ptta_nl_reduce_blocks(rows, c);
+    dim3 grid(nblk, c / 64);
+    launch_k(chan_reduce_kernel<0>, grid, 256, 0, (cudaStream_t)stream, (const bf16*)x, ldx, nullptr, 0, nullptr, 0, nullptr, 0, nullptr, nullptr, rows, c, partial);
+    PTTA_TRY(check_launch("nl_chan_stats"));
+    launch_k(bn_finalize2_sync_kernel, cdiv(c, 32), 1024, 0, (cudaStream_t)stream, partial, nblk, rows, c, gamma, beta, eps, mean, rstd, scale, shift, run_mean,
+                                                                            run_var, num_batches_tracked, momentum, comm->dev, xid);
+    return check_launch("nl_bn_finalize_sync");
+}
+
+int ptta_nl_bn_backward_comm(const void* dy_a, long long ld_a, const void* dy_b, long long ld_b, const void* y, int act, const void* x,
+                             const float* mean, const float* rstd, const float* gamma, float* partial, float* dgamma, float* dbeta, float* coef,
+                             void* dx, void* gskip, long long rows, int c, ptta_comm* comm, int xid, ptta_stream_t stream) {
+    PTTA_CHECK(dy_a && x && mean && rstd && gamma && partial && coef && dx && c % 64 == 0 && rows > 0 && (!act || y), "nl_bn_backward_comm: bad arguments");
+    PTTA_TRY(comm_check(comm, xid, c, "nl_bn_backward_comm"));
+    const int nblk = ptta_nl_reduce_blocks(rows, c);
+    dim3 grid(nblk, c / 64);
+    cudaStream_t st = (cudaStream_t)stream;
+    launch_k(chan_reduce_kernel<1>, grid, 256, 0, st, (const bf16*)x, c, (const bf16*)dy_a, ld_a, (const bf16*)dy_b, ld_b, (const bf16*)y, act, mean, rstd,
+                                               rows, c, partial);
+    PTTA_TRY(check_launch("nl_bn_bwd_reduce"));
+    launch_k(bn_bwd_finalize2_sync_kernel, cdiv(c, 32), 1024, 0, st, partial, nblk, rows, c, gamma, rstd, dgamma, dbeta, coef, coef + c, coef + 2 * c,
+                                                               comm->dev, xid);
+    PTTA_TRY(check_launch("nl_bn_bwd_finalize_sync"));
+    const long long total = (rows * (c / 8) + 1) / 2;
+    launch_k(bn_bwd_apply2_kernel, cdiv(total, 256), 256, 0, st, (const bf16*)dy_a, ld_a, (const bf16*)dy_b, ld_b, (const bf16*)y, act, (const bf16*)x, mean,
+                                                          rstd, coef, coef + c, coef + 2 * c, (bf16*)dx, (bf16*)gskip, rows, c);
+    return check_launch("nl_bn_bwd_apply");
+}
+
 int ptta_nl_add3(const void* a, long long lda, const void* b, long long ldb, const void* c3, long long ldc, void* out, long long rows, int c,
                  ptta_stream_t stream) {
     PTTA_CHECK(a && b && out && c % 64 == 0 && rows > 0, "nl_add3: bad arguments");

@@ -12,6 +12,7 @@
 // Memory-bound kernels: algorithmic bytes = 2 B per element read / written, stated per kernel in DESIGN.md.
 #pragma once
 #include "common.cuh"
+#include "peer_comm.cuh"
 
 namespace ptta {
 
@@ -216,19 +217,11 @@ __device__ __forceinline__ bool partial_sums(const float* __restrict__ partial, 
     return true;
 }
 
-__global__ void __launch_bounds__(1024) bn_finalize2_kernel(const float* __restrict__ partial, int nblk, long long count, int C,
-                                                           const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
-                                                           float* __restrict__ mean, float* __restrict__ rstd, float* __restrict__ scale,
-                                                           float* __restrict__ shift, float* __restrict__ run_mean, float* __restrict__ run_var,
-                                                           long long* __restrict__ nbt, float momentum, float* __restrict__ sums_out) {
-    PDL_SYNC();
-    int c;
-    double s, q;
-    partial += (size_t)blockIdx.y * nblk * 2 * C;                     // statistics group
-    const int go = blockIdx.y * C;
-    mean += go; rstd += go; scale += go; shift += go;
-    if (!partial_sums(partial, nblk, C, c, s, q)) return;
-    if (sums_out) { sums_out[c] = (float)s; return; }          // plain column sums (bias gradients)
+// per channel, from the totals (s, q) = (sum x, sum x^2) over `count` rows
+__device__ __forceinline__ void bn_finalize2_channel(int c, double s, double q, long long count, const float* __restrict__ gamma,
+                                                     const float* __restrict__ beta, float eps, float* __restrict__ mean, float* __restrict__ rstd,
+                                                     float* __restrict__ scale, float* __restrict__ shift, float* __restrict__ run_mean,
+                                                     float* __restrict__ run_var, long long* __restrict__ nbt, float momentum) {
     const double m = s / (double)count;
     double var = q / (double)count - m * m;
     if (var < 0.0) var = 0.0;
@@ -244,6 +237,46 @@ __global__ void __launch_bounds__(1024) bn_finalize2_kernel(const float* __restr
     }
 }
 
+__global__ void __launch_bounds__(1024) bn_finalize2_kernel(const float* __restrict__ partial, int nblk, long long count, int C,
+                                                           const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
+                                                           float* __restrict__ mean, float* __restrict__ rstd, float* __restrict__ scale,
+                                                           float* __restrict__ shift, float* __restrict__ run_mean, float* __restrict__ run_var,
+                                                           long long* __restrict__ nbt, float momentum, float* __restrict__ sums_out) {
+    PDL_SYNC();
+    int c;
+    double s, q;
+    partial += (size_t)blockIdx.y * nblk * 2 * C;                     // statistics group
+    const int go = blockIdx.y * C;
+    mean += go; rstd += go; scale += go; shift += go;
+    if (!partial_sums(partial, nblk, C, c, s, q)) return;
+    if (sums_out) { sums_out[c] = (float)s; return; }          // plain column sums (bias gradients)
+    bn_finalize2_channel(c, s, q, count, gamma, beta, eps, mean, rstd, scale, shift, run_mean, run_var, nbt, momentum);
+}
+
+// shared-model mode (SyncBatchNorm): the same statistics over the batches of ALL ranks -- the rank's (sum x, sum x^2) per channel are
+// exchanged through peer memory (peer_comm.cuh) and added in rank order, count = local rows x world.  Every thread of every block reaches
+// the exchange, so the early exit of the non-owner threads comes after it.  One statistics group (gridDim.y == 1).
+__global__ void __launch_bounds__(1024) bn_finalize2_sync_kernel(const float* __restrict__ partial, int nblk, long long count, int C,
+                                                                const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
+                                                                float* __restrict__ mean, float* __restrict__ rstd, float* __restrict__ scale,
+                                                                float* __restrict__ shift, float* __restrict__ run_mean, float* __restrict__ run_var,
+                                                                long long* __restrict__ nbt, float momentum, const PeerComm comm, int xid) {
+    PDL_SYNC();
+    int c;
+    double s, q;
+    const bool owner = partial_sums(partial, nblk, C, c, s, q);
+    bn_sums_all_ranks(comm, xid, C, owner, c, s, q);
+    if (!owner) return;
+    bn_finalize2_channel(c, s, q, count * comm.world, gamma, beta, eps, mean, rstd, scale, shift, run_mean, run_var, nbt, momentum);
+}
+
+__device__ __forceinline__ void bn_bwd_finalize2_channel(int c, double sg, double sgx, long long count, const float* __restrict__ gamma,
+                                                         const float* __restrict__ rstd, float* __restrict__ k0, float* __restrict__ k1,
+                                                         float* __restrict__ k2) {
+    const float a = gamma[c] * rstd[c];
+    k0[c] = a; k1[c] = (float)((double)a * sg / (double)count); k2[c] = (float)((double)a * sgx / (double)count);
+}
+
 __global__ void __launch_bounds__(1024) bn_bwd_finalize2_kernel(const float* __restrict__ partial, int nblk, long long count, int C,
                                                                const float* __restrict__ gamma, const float* __restrict__ rstd,
                                                                float* __restrict__ dgamma, float* __restrict__ dbeta, float* __restrict__ k0,
@@ -254,8 +287,27 @@ __global__ void __launch_bounds__(1024) bn_bwd_finalize2_kernel(const float* __r
     if (!partial_sums(partial, nblk, C, c, sg, sgx)) return;
     if (dgamma) dgamma[c] = (float)sgx;
     if (dbeta) dbeta[c] = (float)sg;
-    const float a = gamma[c] * rstd[c];
-    k0[c] = a; k1[c] = (float)((double)a * sg / (double)count); k2[c] = (float)((double)a * sgx / (double)count);
+    bn_bwd_finalize2_channel(c, sg, sgx, count, gamma, rstd, k0, k1, k2);
+}
+
+// shared-model mode: d gamma / d beta stay the LOCAL sums (the gradient all-reduce averages them, as DDP does -- the global sums would
+// scale them by the world size); the data gradient uses the means over the global batch (torch SyncBatchNorm backward all-reduces
+// sum_dy / sum_dy_xmu only).  Every thread of every block reaches the exchange.
+__global__ void __launch_bounds__(1024) bn_bwd_finalize2_sync_kernel(const float* __restrict__ partial, int nblk, long long count, int C,
+                                                                    const float* __restrict__ gamma, const float* __restrict__ rstd,
+                                                                    float* __restrict__ dgamma, float* __restrict__ dbeta, float* __restrict__ k0,
+                                                                    float* __restrict__ k1, float* __restrict__ k2, const PeerComm comm, int xid) {
+    PDL_SYNC();
+    int c;
+    double sg, sgx;
+    const bool owner = partial_sums(partial, nblk, C, c, sg, sgx);
+    if (owner) {
+        if (dgamma) dgamma[c] = (float)sgx;
+        if (dbeta) dbeta[c] = (float)sg;
+    }
+    bn_sums_all_ranks(comm, xid, C, owner, c, sg, sgx);
+    if (!owner) return;
+    bn_bwd_finalize2_channel(c, sg, sgx, count * comm.world, gamma, rstd, k0, k1, k2);
 }
 
 // ---- elementwise -----------------------------------------------------------------------------------------------------------------

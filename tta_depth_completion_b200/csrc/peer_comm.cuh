@@ -13,14 +13,21 @@
 //     between two parities, so a fast rank two exchanges ahead never overwrites what a slow rank still reads (it cannot get further
 //     ahead: the exchange in between needs the slow rank's flag).
 //
-// The kernels that spin are tiny (<= 37 blocks), launched on ONE stream in shared mode, so all their blocks are resident.
+// The kernels that spin are small, launched on ONE stream in shared mode, so all their blocks are resident.  The NLSPN entry points
+// enforce PTTA_COMM_MAX_SPIN_BLOCKS (37): a BatchNorm finalize has cdiv(C, 32) <= 32 blocks (C <= 1024, the slot size), the NLSPN
+// flat-buffer Adam 23.
+//
+// Capacity: PTTA_COMM_MAX_XID exchanges per step; one NLSPN step uses 125 (80 BatchNorm forwards: 36 + 36 encoder
+// layers of the real and the zero-image pass, 5 decoder, 3 head; 44 BatchNorm backwards; 1 gradient all-reduce).
 #pragma once
+#include <cuda_runtime.h>
 #include "common.cuh"
 
 namespace ptta {
 
 #define PTTA_COMM_MAX_RANKS 8
-#define PTTA_COMM_MAX_XID 32
+#define PTTA_COMM_MAX_XID 256
+#define PTTA_COMM_MAX_SPIN_BLOCKS 37         // blocks of one spinning kernel (all resident on 148 SMs with the step on one stream)
 #define PTTA_COMM_BN_DOUBLES 2048            // per BatchNorm exchange slot: 2 x up to 1024 channels
 
 struct PeerComm {
@@ -34,7 +41,7 @@ __host__ __device__ inline size_t comm_flags_off() { return 0; }                
 __host__ __device__ inline size_t comm_counters_off() { return (size_t)PTTA_COMM_MAX_XID * PTTA_COMM_MAX_RANKS * 4; }        // uint32 [XID]
 __host__ __device__ inline size_t comm_epoch_off() { return comm_counters_off() + (size_t)PTTA_COMM_MAX_XID * 4; }           // uint32
 __host__ __device__ inline size_t comm_error_off() { return comm_epoch_off() + 4; }                                         // uint32: exchange that timed out + 1
-__host__ __device__ inline size_t comm_data_off() { return 4096; }
+__host__ __device__ inline size_t comm_data_off() { return (comm_error_off() + 4 + 4095) / 4096 * 4096; }                 // 12288
 __host__ __device__ inline size_t comm_bn_slot_off(int parity, int xid) {
     return comm_data_off() + ((size_t)parity * PTTA_COMM_MAX_XID + xid) * PTTA_COMM_BN_DOUBLES * sizeof(double);
 }
@@ -86,10 +93,33 @@ __device__ __forceinline__ void comm_publish_and_wait(const PeerComm& c, int xid
 __device__ __forceinline__ double ld_volatile_f64(const double* p) { return *reinterpret_cast<const volatile double*>(p); }
 __device__ __forceinline__ float ld_volatile_f32(const float* p) { return *reinterpret_cast<const volatile float*>(p); }
 
-// end of a step: the next step's exchanges use the next tag
-__global__ void comm_advance_kernel(PeerComm c) {
-    PDL_SYNC();
-    if (threadIdx.x == 0 && blockIdx.x == 0) *reinterpret_cast<volatile uint32_t*>(c.base[c.rank] + comm_epoch_off()) += 1u;
+// sums of one BatchNorm call over ALL ranks (SyncBatchNorm semantics of the shared-model mode): the owner threads publish the rank's
+// (sum, sum of squares) / (sum dy, sum dy xhat) per channel, wait for every rank, and add the ranks' values in rank order.  Called by
+// ALL threads of ALL blocks of the kernel (comm_publish_and_wait is a rendezvous); C <= PTTA_COMM_BN_DOUBLES / 2.
+__device__ __forceinline__ void bn_sums_all_ranks(const PeerComm& comm, int xid, int C, bool owner, int ch, double& a, double& b) {
+    const uint32_t tag = comm_tag(comm);
+    const size_t off = comm_bn_slot_off((int)(tag & 1u), xid);
+    if (owner) {
+        double* slot = reinterpret_cast<double*>(comm.base[comm.rank] + off);
+        slot[ch] = a; slot[C + ch] = b;
+    }
+    comm_publish_and_wait(comm, xid, tag);
+    if (owner) {
+        a = 0.0; b = 0.0;
+        for (int r = 0; r < comm.world; ++r) {
+            const double* slot = reinterpret_cast<const double*>(comm.base[r] + off);
+            a += ld_volatile_f64(slot + ch); b += ld_volatile_f64(slot + C + ch);
+        }
+    }
 }
 
 }  // namespace ptta
+
+// host handle of the C ABI (include/ptta_b200.h `ptta_comm_*`): the device-side view every engine entry point passes to its kernels,
+// the local block and the peers' mapped blocks
+struct ptta_comm {
+    ptta::PeerComm dev;
+    void* local = nullptr;
+    void* opened[PTTA_COMM_MAX_RANKS] = {};
+    size_t bytes = 0;
+};

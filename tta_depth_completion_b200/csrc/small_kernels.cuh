@@ -1111,25 +1111,6 @@ __device__ __forceinline__ void stats_fused_finalize(const StatsFin& fin, const 
     }
 }
 
-// sums of one BatchNorm call over ALL ranks (SyncBatchNorm semantics of the shared-model mode): the owner threads publish the rank's
-// (sum, sum of squares) / (sum dy, sum dy xhat) per channel, wait for every rank, and add the ranks' values in rank order
-__device__ __forceinline__ void bn_sums_all_ranks(const PeerComm& comm, int xid, int C, bool owner, int ch, double& a, double& b) {
-    const uint32_t tag = comm_tag(comm);
-    const size_t off = comm_bn_slot_off((int)(tag & 1u), xid);
-    if (owner) {
-        double* slot = reinterpret_cast<double*>(comm.base[comm.rank] + off);
-        slot[ch] = a; slot[C + ch] = b;
-    }
-    comm_publish_and_wait(comm, xid, tag);
-    if (owner) {
-        a = 0.0; b = 0.0;
-        for (int r = 0; r < comm.world; ++r) {
-            const double* slot = reinterpret_cast<const double*>(comm.base[r] + off);
-            a += ld_volatile_f64(slot + ch); b += ld_volatile_f64(slot + C + ch);
-        }
-    }
-}
-
 __global__ void __launch_bounds__(FIN_THREADS) bn_finalize_kernel(const double* __restrict__ partial, int nblk, long long count, int C, BnParams p, int training,
                                                                   const PeerComm comm, int xid) {
     PDL_SYNC();
@@ -1588,6 +1569,12 @@ __global__ void __launch_bounds__(256) adam_kernel(const AdamChunk* __restrict__
 }
 __global__ void adam_advance_kernel(AdamHyper* hy) {
     PDL_SYNC(); hy->step += 1; }
+
+// end of a step: the next step's exchanges use the next tag
+__global__ void comm_advance_kernel(PeerComm c) {
+    PDL_SYNC();
+    if (threadIdx.x == 0 && blockIdx.x == 0) *reinterpret_cast<volatile uint32_t*>(c.base[c.rank] + comm_epoch_off()) += 1u;
+}
 
 // Shared-model mode: mean all-reduce of the adapted-parameter gradients FUSED with the Adam update, one launch, one-shot over NVLink
 // peer memory.  Block = one chunk of the chunk table (as adam_kernel): it copies its part of the local gradient into the rank's slot, the

@@ -650,6 +650,10 @@ class ExternalModel_Adapt(object):
                 # the network must see the NORMALISED image and the smoothness loss the raw one (src/tta_main.py:595-620): without the folded
                 # normalisation the fused step would feed the raw image to both
                 raise RuntimeError('NLSPN tta_step: call set_image_normalization(scale, shift) first (ImageNet statistics folded into the stem)')
+            comm = getattr(self.model, '_comm', None)
+            if comm is not None:             # shared-model mode: every rank must step on the same (N, H, W) (SyncBatchNorm count)
+                from .sharding import check_same_shape
+                check_same_shape(comm, (image_raw.shape[0], image_raw.shape[2], image_raw.shape[3]))
             eng.set_image_normalization(self.model.img_scale, self.model.img_shift)
             eng.tta_step(image_raw, image_raw, sparse_depth, learning_rate, w_loss_sparse_depth, w_loss_smoothness, w_loss_cos,
                          self.max_input_depth, graph=graph, betas=betas, eps=eps, weight_decay=weight_decay)

@@ -89,6 +89,43 @@ class NlspnEngine:
         self._adam_host = None
         self.adam_step_dev = share_from.adam_step_dev if share_from is not None else torch.zeros(1, dtype=torch.int32, device=self.dev)
         self._graph, self._graph_key, self._seen_key = None, None, None
+        # shared-model mode (set_comm): exchanges of the running step body, in issue order
+        self._comm, self._syncing, self._next_xid, self._exchange_at_world1 = None, False, 0, False
+        if share_from is not None and share_from._comm is not None:
+            self.set_comm(share_from._comm, share_from._exchange_at_world1)
+
+    # ---- shared-model mode ----------------------------------------------------------------------------------------------------------
+    def set_comm(self, comm, exchange_at_world1=False):
+        """Join the peer communicator of the shared-model mode (sharding.PeerCommunicator; None: leave it).  With comm.world > 1 the
+        TRAINING step takes every train-mode BatchNorm's statistics over all ranks (SyncBatchNorm: forward sums and backward sums
+        exchanged inside the finalize kernels) and mean-all-reduces the flat gradient buffer inside the Adam kernel, so every rank applies
+        the same update.  The eval forward keeps local statistics (SyncBatchNorm does not synchronise in eval mode).  The step then runs
+        on ONE stream: the exchanging kernels spin until every rank has arrived, so all their blocks must be resident, and every rank
+        must issue its exchanges in the same order.
+        exchange_at_world1: a one-rank communicator runs the exchanging kernels too (otherwise world 1 is the plain step).  With one rank
+        the rank-order sums are 0 + the local sums and the count is rows x 1, so the step computes what the plain step computes; this
+        runs the rendezvous, the epoch advance and the slot parities on a single GPU."""
+        self._exchange_at_world1 = bool(exchange_at_world1)
+        if comm is not None and (comm.world > 1 or self._exchange_at_world1):
+            if self.merge_branches:
+                raise NotImplementedError('NLSPN shared-model mode: merge_branches (batch-2N encoder) has no SyncBatchNorm form')
+            if comm.grad_floats < self.flat_g.numel():
+                raise RuntimeError('NLSPN shared-model mode: the communicator holds %d gradient floats, the model has %d'
+                                   % (comm.grad_floats, self.flat_g.numel()))
+        self._comm = comm
+        self._graph, self._graph_key, self._seen_key = None, None, None
+
+    def _shared(self):
+        return self._comm is not None and (self._comm.world > 1 or self._exchange_at_world1)
+
+    def _take_xid(self):
+        """exchange ids in issue order, reset at the start of every step body (the same sequence on every rank; a captured graph keeps
+        them, the tags come from the device-side epoch)"""
+        xid = self._next_xid
+        if xid >= _lib.lib().ptta_comm_max_exchanges():
+            raise RuntimeError('NLSPN shared-model mode: more than %d peer exchanges in one step' % _lib.lib().ptta_comm_max_exchanges())
+        self._next_xid += 1
+        return xid
 
     # ---- parameters -------------------------------------------------------------------------------------------------------------
     def _build_flat(self, sd):
@@ -235,8 +272,13 @@ class NlspnEngine:
             self.bn_state[bn] = st
         rm, rv, nbt = running if running is not None else (None, None, None)
         partial = self.partial_z if bn.startswith('z.') else self.partial
-        check(_lib.lib().ptta_nl_bn_stats(ptr(x), c, rows, c, ptr(gamma), ptr(beta), BN_EPS, ptr(partial), ptr(st['mean']), ptr(st['rstd']),
-                                          ptr(st['scale']), ptr(st['shift']), ptr(rm), ptr(rv), ptr(nbt), 0.1, _stream()), 'nl_bn_stats')
+        if self._syncing:
+            check(_lib.lib().ptta_nl_bn_stats_comm(ptr(x), c, rows, c, ptr(gamma), ptr(beta), BN_EPS, ptr(partial), ptr(st['mean']), ptr(st['rstd']),
+                                                   ptr(st['scale']), ptr(st['shift']), ptr(rm), ptr(rv), ptr(nbt), 0.1, self._comm.handle,
+                                                   self._take_xid(), _stream()), 'nl_bn_stats_comm')
+        else:
+            check(_lib.lib().ptta_nl_bn_stats(ptr(x), c, rows, c, ptr(gamma), ptr(beta), BN_EPS, ptr(partial), ptr(st['mean']), ptr(st['rstd']),
+                                              ptr(st['scale']), ptr(st['shift']), ptr(rm), ptr(rv), ptr(nbt), 0.1, _stream()), 'nl_bn_stats')
         self.launches += 2
         return st
 
@@ -265,11 +307,17 @@ class NlspnEngine:
             dg, db = self.grads[bn_key + '.weight'], self.grads[bn_key + '.bias']
         dx = self.buf(out_name, x.shape)
         gskip = self.buf(gskip_name, x.shape) if gskip_name else None
-        check(_lib.lib().ptta_nl_bn_backward(ptr(dy_a), ld_a, ptr(dy_b), ld_b, ptr(y), act, ptr(x), ptr(st['mean']), ptr(st['rstd']), ptr(gamma),
-                                             ptr(self.partial), ptr(dg), ptr(db), ptr(self.coef), ptr(dx), ptr(gskip), rows, c, _stream()),
-              'nl_bn_backward')
-        self.launches += 3
+        self._bn_backward_call(dy_a, ld_a, dy_b, ld_b, y, act, x, st, gamma, dg, db, dx, gskip, rows, c)
         return dx, gskip
+
+    def _bn_backward_call(self, dy_a, ld_a, dy_b, ld_b, y, act, x, st, gamma, dg, db, dx, gskip, rows, c):
+        args = (ptr(dy_a), ld_a, ptr(dy_b), ld_b, ptr(y), act, ptr(x), ptr(st['mean']), ptr(st['rstd']), ptr(gamma), ptr(self.partial), ptr(dg), ptr(db),
+                ptr(self.coef), ptr(dx), ptr(gskip), rows, c)
+        if self._syncing:
+            check(_lib.lib().ptta_nl_bn_backward_comm(*args, self._comm.handle, self._take_xid(), _stream()), 'nl_bn_backward_comm')
+        else:
+            check(_lib.lib().ptta_nl_bn_backward(*args, _stream()), 'nl_bn_backward')
+        self.launches += 3
 
     # ---- forward ----------------------------------------------------------------------------------------------------------------
     def set_image_normalization(self, scale, shift):
@@ -438,7 +486,10 @@ class NlspnEngine:
         # packed weights: they run on a second stream, concurrently with the real branch (fork / join through events, also inside a
         # CUDA-graph capture); their small layers fill the SMs the real branch's small layers leave idle
         main = torch.cuda.current_stream()
-        side = self.side_stream if self.two_streams else main
+        # shared-model mode: one stream (the exchanging kernels of the two branches must not wait on each other across streams)
+        side = self.side_stream if (self.two_streams and not self._syncing) else main
+        if self._syncing and self.merge_branches:
+            raise NotImplementedError('NLSPN shared-model mode: merge_branches (batch-2N encoder) has no SyncBatchNorm form')
         if self.merge_branches and image is not None:
             fe_m = self.encoder_merged(image, sparse_depth)
             fe = [t[:self.N] for t in fe_m]
@@ -532,9 +583,7 @@ class NlspnEngine:
         st = self.bn_state['r.dec1']
         dF = self.buf('g.dec1.raw', (N, H, W, 192))
         rows = N * H * W
-        check(L.ptta_nl_bn_backward(ptr(dcat1), 256, None, 0, ptr(B['r.dec1.act']), ACT_LEAKY, ptr(B['r.dec1.raw']), ptr(st['mean']), ptr(st['rstd']),
-                                    ptr(gw), ptr(self.partial), ptr(dgw), ptr(dgb), ptr(self.coef), ptr(dF), None, rows, 192, _stream()), 'nl_bn_backward')
-        self.launches += 3
+        self._bn_backward_call(dcat1, 256, None, 0, B['r.dec1.act'], ACT_LEAKY, B['r.dec1.raw'], st, gw, dgw, dgb, dF, None, rows, 192)
         dcat2 = self.conv('dec1.d', dF, out_name='g.cat2', hw=(H, W))                                  # [N,H,W,128] = d(fd2 | fe2)
         # decoder: dec2 .. dec5
         d2, _ = self.bn_backward('r.', 'dec2.1', dcat2, 128, None, 0, B['r.dec2.1.act'], ACT_LEAKY, B['r.dec2.raw'], 'g.dec2.raw')
@@ -614,8 +663,14 @@ class NlspnEngine:
 
     def adam_step(self):
         self.step_count += 1
-        check(_lib.lib().ptta_adam_flat_dev(ptr(self.flat_p), ptr(self.flat_g), ptr(self.flat_m), ptr(self.flat_v), self.flat_p.numel(),
-                                            ptr(self.adam_hyper), ptr(self.adam_step_dev), _stream()), 'adam_flat_dev')
+        if self._syncing:
+            # gradient mean all-reduce fused with the update; the averaged gradient is left in flat_g (DDP's .grad)
+            check(_lib.lib().ptta_adam_flat_dev_comm(ptr(self.flat_p), ptr(self.flat_g), ptr(self.flat_m), ptr(self.flat_v), self.flat_p.numel(),
+                                                     ptr(self.adam_hyper), ptr(self.adam_step_dev), self._comm.handle, self._take_xid(), _stream()),
+                  'adam_flat_dev_comm')
+        else:
+            check(_lib.lib().ptta_adam_flat_dev(ptr(self.flat_p), ptr(self.flat_g), ptr(self.flat_m), ptr(self.flat_v), self.flat_p.numel(),
+                                                ptr(self.adam_hyper), ptr(self.adam_step_dev), _stream()), 'adam_flat_dev')
         self.repack_adapted()
         self.launches += 3
 
@@ -649,6 +704,18 @@ class NlspnEngine:
         self.step_count += 1
 
     def _step_body(self, image_norm, image_raw, sparse_depth, w_sd, w_sm, w_cos, cap):
+        if not self._shared():
+            return self._step_kernels(image_norm, image_raw, sparse_depth, w_sd, w_sm, w_cos, cap)
+        self._syncing, self._next_xid = True, 0
+        try:
+            self._step_kernels(image_norm, image_raw, sparse_depth, w_sd, w_sm, w_cos, cap)
+        finally:
+            self._syncing = False
+        check(_lib.lib().ptta_comm_advance(self._comm.handle, _stream()), 'comm_advance')       # the next step's exchanges use the next tag
+        self.launches += 1
+        self.exchanges_per_step = self._next_xid
+
+    def _step_kernels(self, image_norm, image_raw, sparse_depth, w_sd, w_sm, w_cos, cap):
         N, H, W = self.N, self.H, self.W
         d_f = self.buf('filtered_depth', (N, 1, H, W), torch.float32)
         v_f = self.buf('filtered_validity', (N, 1, H, W), torch.float32)

@@ -154,6 +154,7 @@ class NLSPNModel_Adapt(object):
         self._adapt_names = []
         self._param_objs = OrderedDict()
         self._syncbn = False                     # set by convert_syncbn()
+        self._comm = None                        # shared-model mode (sharding.enable_shared_model): every engine joins it
 
     # -- construction ---------------------------------------------------------------------------------------------------------------
     def _prepare_head(self, mode):
@@ -182,7 +183,14 @@ class NLSPNModel_Adapt(object):
                 self._sd = eng.sd                      # device tensors; adapted entries are views of the engine's flat buffer
                 self._param_objs = OrderedDict((k, torch.nn.Parameter(eng.params[k], requires_grad=True)) for k in self._adapt_names)
             self._engines[key] = eng
+        if self._comm is not None and eng._comm is not self._comm:
+            eng.set_comm(self._comm)
         return eng
+
+    def _refuse_shared(self, what):
+        if self._comm is not None:
+            raise RuntimeError('NLSPN %s on a shared model (sharding.enable_shared_model): this path has no SyncBatchNorm / gradient '
+                               'all-reduce form and would mix local and global semantics; use sharding.shared_model_step' % what)
 
     def _materialise(self, n=1, h=32, w=32):
         """parameters exist only once an engine does: create the smallest one if the driver asks for them before the first frame"""
@@ -200,6 +208,7 @@ class NLSPNModel_Adapt(object):
             raise NotImplementedError('NLSPN native back-end: forward(loss_type=%r) -- stage 2 runs as the fused `head_step` '
                                       '(nlspn_prepare.NlspnHeadTrainer), stage 1 is not built' % (loss_type,))
         if self.training and 'adapt' in loss_type:
+            self._refuse_shared('autograd adaptation forward')
             self._materialise(image.shape[0], image.shape[2], image.shape[3])
             return _NlspnForwardFn.apply(self, image, sparse_depth, *self._param_objs.values())
         eng = self._engine_for(image)
@@ -267,6 +276,7 @@ class NLSPNModel_Adapt(object):
                   img_scale=None, img_shift=None, graph=False):
         """One whole stage-2 step (src/head_main.py:437-480) through the library; `image` is the network input unless a normalisation is folded
         into the stem (img_scale / img_shift)."""
+        self._refuse_shared('head_step (stage 2)')
         tr = self._head_trainer_for(image)
         tr.eng.set_image_normalization(img_scale, img_shift)
         tr.head_step(image, sparse_depth, learning_rate, betas, eps, weight_decay, max_input_depth=max_input_depth, graph=graph)

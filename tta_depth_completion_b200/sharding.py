@@ -8,7 +8,8 @@ Optional mode ("shared"): every rank holds the same model and processes its own 
 over all ranks (SyncBatchNorm) and the adapted-parameter gradients (one flat fp32 buffer, 74 080 floats = 296 KB for MSG-CHN
 `2layers`) are mean-all-reduced before the Adam step, so all replicas apply the identical update (the reference: SyncBN + DDP over all
 1.53 M gradients, src/msg_chn_model_adapt.py:480,555-556).  Both exchanges are one-shot reads of NVLink peer memory inside the engine's own
-kernels (csrc/peer_comm.cuh): the all-reduce is FUSED with the Adam update, the step stays one CUDA graph, no NCCL call on the path."""
+kernels (csrc/peer_comm.cuh): the all-reduce is FUSED with the Adam update, the step stays one CUDA graph, no NCCL call on the path.
+The NLSPN back-end has the same mode (its ~46 K-float flat gradient buffer, 125 exchanges per step; INTEGRATION.md section 2f)."""
 import torch
 import torch.distributed as dist
 
@@ -46,6 +47,8 @@ class PeerCommunicator:
         self.L = _lib.lib()
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
+        self.group, self.grad_floats = group, int(grad_floats)
+        self.checked_shapes = set()          # input shapes all ranks were found to share (NLSPN: check_same_shape)
         if device is not None and torch.device(device).index is not None:
             torch.cuda.set_device(device)
         handle = c_void_p()
@@ -80,10 +83,16 @@ class PeerCommunicator:
 
 
 def enable_shared_model(model, group=None):
-    """Switch a MSG-CHN `ExternalModel_Adapt` to the shared-model mode: every engine it creates from now on (and the ones it has)
+    """Switch a MSG-CHN or NLSPN `ExternalModel_Adapt` to the shared-model mode: every engine it creates from now on (and the ones it has)
     exchanges its train-mode BatchNorm sums and its adapted-parameter gradients with the other ranks through peer memory, so all ranks
     apply the identical update -- the reference's DDP + SyncBatchNorm semantics (src/msg_chn_model_adapt.py:480,555-556) without a
-    collective call on the path.  Returns the communicator (keep it alive)."""
+    collective call on the path.  Returns the communicator (keep it alive).
+
+    NLSPN: convert_syncbn() must have been called (the reference driver always does, src/tta_main.py:327; without it the reference's
+    BatchNorms would stay local).  The training step (shared_model_step, tta_step) then runs on one stream; the autograd path and the
+    stage-2 head_step raise on a shared model."""
+    if getattr(model, 'model_name', None) == 'nlspn':
+        return _enable_shared_nlspn(model, group)
     wrapper = model.model
     comm = PeerCommunicator(wrapper._flat['grad'].numel(), group=group, device=wrapper.device)
     wrapper._comm = comm
@@ -92,12 +101,45 @@ def enable_shared_model(model, group=None):
     return comm
 
 
+def _enable_shared_nlspn(model, group):
+    wrapper = model.model
+    if not wrapper._syncbn:
+        raise RuntimeError('NLSPN shared-model mode needs convert_syncbn() first: without it the reference\'s BatchNorms are local and '
+                           'adapt_parameters(\'meta_bn\') hands a different tensor set to the optimiser')
+    base = wrapper._materialise()
+    comm = PeerCommunicator(base.flat_g.numel(), group=group, device=wrapper.device)
+    wrapper._comm = comm
+    for eng in wrapper._engines.values():
+        eng.set_comm(comm)
+    return comm
+
+
+def check_same_shape(comm, shape):
+    """Once per new input shape (called by the NLSPN tta_step of a shared model): every rank of the communicator must step on the same (N, H, W) -- the SyncBatchNorm count is local rows x
+    world, and the ranks' exchange sequences must match.  One host all_gather_object; raises on a mismatch."""
+    shape = tuple(int(v) for v in shape)
+    if comm.world == 1 or shape in comm.checked_shapes:
+        return
+    shapes = [None] * comm.world
+    dist.all_gather_object(shapes, shape, group=comm.group)
+    if any(tuple(s) != shape for s in shapes):
+        raise RuntimeError('shared-model mode: the ranks step on different input shapes %s (unequal per-rank batches are not supported)' % (shapes,))
+    comm.checked_shapes.add(shape)
+
+
 def shared_model_step(model, image_raw, sparse_depth, learning_rate, w_sd=1.0, w_sm=1.0, w_cos=0.1, group=None, graph=False):
     """One shared-model adaptation step.  With a peer communicator (enable_shared_model) this is the engine's ordinary fused step -- the
     exchanges happen inside its kernels and the step replays from a CUDA graph.  Without one (CPU tensors / gloo tests, or
     `PTTA_SHARED_NCCL=1`): local forward / loss / backward, mean all-reduce of the flat gradient buffer through torch.distributed,
     fused Adam -- local BatchNorm statistics, the round-1 form."""
     wrapper = model.model
+    if getattr(model, 'model_name', None) == 'nlspn':
+        # NLSPN: the engine's fused step with the exchanges inside its kernels (eager, or replayed from a CUDA graph)
+        comm = getattr(wrapper, '_comm', None)
+        if comm is None:
+            raise RuntimeError('NLSPN shared_model_step: call sharding.enable_shared_model(model) first')
+        model.tta_step(image_raw, sparse_depth, learning_rate, w_sd, w_sm, w_cos, graph=graph)
+        return
     eng = wrapper._engine_for(image_raw)
     comm = getattr(wrapper, '_comm', None)
     if comm is not None:
