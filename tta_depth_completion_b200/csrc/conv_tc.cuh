@@ -34,8 +34,14 @@ struct ConvTcParams {
 };
 
 
+// Shared-memory layout per instantiation (MASK / ADDS / UP2: the epilogue operands, see conv3x3_tc_body).  The plain kernel spends
+// it all on eight input-row slots and the two output staging tiles; the operand instantiations give up input-row slots, and the
+// mask (data-gradient) ones the out2 tile they never write, for the operand rings the producer fills by TMA.
+template <bool MASK = false, bool ADDS = false, bool UP2 = false>
 struct ConvTcCfg {
-    static const int RB = 8;                      // input-row slots in the shared-memory ring
+    static const int NOPS = (MASK ? 1 : 0) + (ADDS ? 1 : 0);     // full-resolution operand maps (mask, add / add2)
+    static const bool OUT2 = !MASK;               // the out2 staging tile exists
+    static const int RB = (NOPS == 0 && !UP2) || (MASK && !ADDS) ? 8 : (UP2 && ADDS ? 4 : 6);   // input-row slots in the shared-memory ring
     static const int NSLOT = 8;                   // output-row accumulator slots per pixel parity (2 x 8 x 32 columns = all 512)
     static const int BOXP = 130;                  // pixel PAIRS per staged row (128 + one halo pair each side)
     static const int ROW_BYTES = BOXP * 128;      // 16640: what one TMA box delivers
@@ -43,9 +49,19 @@ struct ConvTcCfg {
     static const int W_BYTES = 9 * 32 * 64;       // 18432
     static const int OUT_TILE = 4096;             // one TMEM lane quarter's output row: 32 pixel pairs x 128 B (one TMA store box)
     static const int STAGE_BYTES = 4 * 2 * OUT_TILE;   // per output map: 4 quarters x double buffer
+    static const int OP_BYTES = 128 * 128;        // one operand's row of a strip: 128 pixel pairs x 128 B (one SWIZZLE_128B box)
+    static const int OPD = NOPS ? 2 : 0;          // operand ring: output rows in flight
+    static const int UP_BOX = 130;                // half-resolution pixels per staged row: a strip's low-resolution span (<= 129) + 1
+    static const int UP_BYTES = UP_BOX * 64;      // 8320 (SWIZZLE_64B box)
+    static const int UP_SLOT = 9216;              // UP_BYTES rounded up to 1024 B
+    static const int UPD = UP2 ? 4 : 0;           // up2 ring: half-resolution rows in flight (an output row reads two)
+    static const int LAG = RB - 2;                // the producer stages output row y's operands right after input row y + LAG
     static const int BAR_BYTES = 1024;
-    static const int SMEM = 1024 /*align slack*/ + RB * SLOT_BYTES + W_BYTES + 2 * STAGE_BYTES + BAR_BYTES;
+    static const int SMEM = 1024 /*align slack*/ + RB * SLOT_BYTES + W_BYTES + (OUT2 ? 2 : 1) * STAGE_BYTES + OPD * NOPS * OP_BYTES +
+                            UPD * UP_SLOT + BAR_BYTES;
     static const int THREADS = 320;               // warp 0 TMA producer | warp 1 MMA issuer | warps 2-9 epilogue (2 per TMEM lane quarter)
+    static_assert(SMEM <= 232448, "conv3x3_tc: shared memory over the 227 KB a block can opt into");
+    static_assert(!(MASK && UP2), "conv3x3_tc: mask and up2 are never used together");
 };
 
 // one bit per bf16 of a 16 B chunk: value > 0
@@ -106,35 +122,6 @@ __global__ void pack_conv_weight_tc_kernel(const bf16* __restrict__ pack, bf16* 
     *reinterpret_cast<uint4*>(reinterpret_cast<unsigned char*>(image) + row * 64 + ((c ^ ((row >> 1) & 3)) << 4)) = v;
 }
 
-// The epilogue thread of lane l needs its OWN pixel's 64 B (pair l of the quarter, parity `par`) of an NHWC operand row.  Loading them
-// directly (lane l reads 4 x 16 B at a 128 B stride between lanes) makes every request touch 32 cache lines: with mask and add operands
-// the LSU, not HBM, then sets the row time (measured 24 / 30 us against 14 us without operands).  Instead lane l loads chunk (l & 3) of
-// pair 8 j + (l >> 2), j = 0..3 -- four lanes cover one pixel's 64 contiguous bytes, 8 lines per request -- and the values are
-// transposed back with warp shuffles: chunk g of pair l sits in load j = l >> 3 of lane 4 (l & 7) + g.
-struct OperandRows { uint4 r[4]; };
-__device__ __forceinline__ void operand_rows_load(OperandRows& o, const bf16* base /* pixel xw + par of the row */, int vp, int lane, bool nc_load) {
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const int pair = j * 8 + (lane >> 2);
-        const uint4* src = reinterpret_cast<const uint4*>(base + (size_t)pair * 64) + (lane & 3);
-        o.r[j] = pair < vp ? (nc_load ? __ldg(src) : *src) : make_uint4(0u, 0u, 0u, 0u);
-    }
-}
-__device__ __forceinline__ void operand_rows_transpose(const OperandRows& o, int lane, uint4 (&out)[4]) {
-    const int jd = lane >> 3;
-#pragma unroll
-    for (int g = 0; g < 4; ++g) {
-        const int src = ((lane & 7) << 2) + g;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            uint4 t;
-            t.x = __shfl_sync(0xffffffffu, o.r[j].x, src); t.y = __shfl_sync(0xffffffffu, o.r[j].y, src);
-            t.z = __shfl_sync(0xffffffffu, o.r[j].z, src); t.w = __shfl_sync(0xffffffffu, o.r[j].w, src);
-            if (j == jd) out[g] = t;
-        }
-    }
-}
-
 // Scatter-form implicit GEMM over PIXEL PAIRS.
 //
 // Shared-memory / TMA view of the NHWC bf16 input: [N][H][W/2][64] -- one 128 B row per pixel pair, SWIZZLE_128B, the layout
@@ -155,10 +142,18 @@ __device__ __forceinline__ void operand_rows_transpose(const OperandRows& o, int
 //
 // Roles: warp 0 TMA producer (one box per input row) | warp 1 MMA issuer (warp stays converged, elect.sync issues) |
 // warps 2-9 epilogue, two per TMEM lane quarter (one takes the even-pixel accumulator bank, one the odd): tcgen05.ld ->
-// bias / derivative mask / add / ReLU in registers (mask and add are the thread's own 64 contiguous bytes, prefetched before
-// the accumulator wait) -> bf16 -> the pixel's half of its 128 B pair row in a SWIZZLE_128B staging tile -> one TMA store per
-// quarter row (32 pairs x 128 B; the tensor map clips the ragged right edge), double buffered.  Every mbarrier has one
-// arrival per phase except slot_empty (one per epilogue warp).
+// bias / derivative mask / add / ReLU in registers -> bf16 -> the pixel's half of its 128 B pair row in a SWIZZLE_128B staging
+// tile -> one TMA store per quarter row (32 pairs x 128 B; the tensor map clips the ragged right edge), double buffered.
+//
+// Epilogue operands come through shared memory, staged by the producer warp with TMA:
+//   mask / add / add2: per output row one box of 128 pixel pairs of each map, in the same pair-row view and swizzle as the output
+//   staging tile, into a ring of OPD output rows (zero-filled right of the image).  The thread's pixel sits at the address it
+//   writes its output to, so the reads need no shuffles and hit no bank conflicts.  `add` may alias `out` (in-place accumulate):
+//   a CTA's TMA load of a row completes before its epilogue stores that row, and no other CTA touches the row.
+//   up2: the half-resolution rows the strip's output rows read (align_corners = True), 130 pixels from the strip's first source
+//   column, in a ring of UPD rows keyed by half-resolution row: each is read from global memory once per segment.
+// The producer stages output row y's operands after it issued input row y + LAG, so it can still run LAG rows ahead of the MMA.
+// Every mbarrier has one arrival per phase except slot_empty, op_empty and up_empty (one per epilogue warp).
 __device__ __forceinline__ void conv_tc_pixel(const uint32_t (&v)[32], const float (&bias)[32], const uint4* mk, const uint4* ad, int relu_out,
                                               uint4 (&ov)[4], const float* up = nullptr, uint4* ov_pre = nullptr) {
     float f[32];
@@ -215,11 +210,6 @@ __device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, uint32_t sr
     asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
                  ::"l"(map), "r"(src), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
 }
-// L2 prefetch of a contiguous global range (bytes: multiple of 16): issued by the producer several rows ahead of the epilogue warps that
-// read the data with plain loads (mask / add rows), so those loads find the lines in L2 instead of paying the DRAM latency per row
-__device__ __forceinline__ void l2_prefetch(const void* gptr, uint32_t bytes) {
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(gptr), "r"(bytes) : "memory");
-}
 __device__ __forceinline__ void bulk_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_store_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void bulk_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
@@ -232,8 +222,9 @@ __device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t threads) { 
 // kernel sits at its register cap (168 with 10 warps): every operand path compiled in costs the plain forward conv registers it never uses.
 template <int NC, bool MASK, bool ADDS, bool UP2>
 __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, const CUtensorMap& tmap_out, const CUtensorMap& tmap_out2,
+                                                const CUtensorMap& tmap_mask, const CUtensorMap& tmap_add, const CUtensorMap& tmap_up,
                                                 const ConvTcParams& p) {
-    typedef ConvTcCfg C;
+    typedef ConvTcCfg<MASK, ADDS, UP2> C;
     constexpr uint32_t W_BYTES_NC = 9 * NC * 64;
     extern __shared__ unsigned char smem_raw[];
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -241,22 +232,32 @@ __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, cons
     const uint32_t rows_s = smem_base;                                   // RB row slots
     const uint32_t w_s = smem_base + C::RB * C::SLOT_BYTES;              // weights, SW64 canonical, row = kx*96 + (2-ky)*32 + cout
     const uint32_t stage_s = w_s + C::W_BYTES;                           // `out` staging: [quarter][2][32 pairs x 128 B], then `out2`
-    const uint32_t bar_s = stage_s + 2 * C::STAGE_BYTES;
+    const uint32_t op_s = stage_s + (C::OUT2 ? 2 : 1) * C::STAGE_BYTES;  // [OPD][mask | add][128 pairs x 128 B]
+    const uint32_t up_s = op_s + C::OPD * C::NOPS * C::OP_BYTES;         // [UPD][130 half-resolution pixels x 64 B]
+    const uint32_t bar_s = up_s + C::UPD * C::UP_SLOT;
     const uint32_t row_full = bar_s;                         // [RB]    TMA     -> MMA       (expect_tx + complete_tx)
     const uint32_t row_free = bar_s + 8 * C::RB;             // [RB]    MMA     -> producer  (tcgen05.commit)
     const uint32_t slot_full = bar_s + 16 * C::RB;           // [NSLOT] MMA     -> epilogue  (tcgen05.commit)
     const uint32_t slot_empty = slot_full + 8 * C::NSLOT;    // [NSLOT] epilogue -> MMA      (8 arrivals: one per epilogue warp)
     const uint32_t w_full = slot_empty + 8 * C::NSLOT;       //         bulk copy of the weight image landed
     const uint32_t tmem_slot = w_full + 8;                   // u32
+    const uint32_t op_full = tmem_slot + 8;                  // [OPD]   TMA     -> epilogue  (expect_tx + complete_tx)
+    const uint32_t op_empty = op_full + 8 * C::OPD;          // [OPD]   epilogue -> producer (8 arrivals)
+    const uint32_t up_full = op_empty + 8 * C::OPD;          // [UPD]   TMA     -> epilogue
+    const uint32_t up_empty = up_full + 8 * C::UPD;          // [UPD]   epilogue -> producer (8 arrivals)
     volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(smem + (tmem_slot - smem_base));
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int uh2 = p.H >> 1, uw2 = p.W >> 1;                // up2: half-resolution size
 
     // ---- one-time set-up: overlaps the tail of the previous kernel (programmatic dependent launch) --------------------
     if (warp == 0 && lane == 0) {
         tc::prefetch_tmap(&tmap_in);
         tc::prefetch_tmap(&tmap_out);
         tc::prefetch_tmap(&tmap_out2);
+        if (MASK) tc::prefetch_tmap(&tmap_mask);
+        if (ADDS) tc::prefetch_tmap(&tmap_add);
+        if (UP2) tc::prefetch_tmap(&tmap_up);
         for (int i = 0; i < C::RB; ++i) {
             tc::mbar_init(row_full + 8 * i, 1);
             tc::mbar_init(row_free + 8 * i, 1);
@@ -264,6 +265,14 @@ __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, cons
         for (int i = 0; i < C::NSLOT; ++i) {
             tc::mbar_init(slot_full + 8 * i, 1);
             tc::mbar_init(slot_empty + 8 * i, 8);
+        }
+        for (int i = 0; i < C::OPD; ++i) {
+            tc::mbar_init(op_full + 8 * i, 1);
+            tc::mbar_init(op_empty + 8 * i, 8);
+        }
+        for (int i = 0; i < C::UPD; ++i) {
+            tc::mbar_init(up_full + 8 * i, 1);
+            tc::mbar_init(up_empty + 8 * i, 8);
         }
         tc::mbar_init(w_full, 1);
         tc::fence_barrier_init();
@@ -287,26 +296,56 @@ __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, cons
                          ::"r"(w_s), "l"(p.w), "r"(W_BYTES_NC), "r"(w_full) : "memory");
         }
         __syncwarp();
-        uint32_t r = 0;
+        uint32_t r = 0, o = 0, u = 0;            // input rows, operand rows, half-resolution rows staged so far
         for (int lin = lin0; lin < lin1;) {
             const int col = lin / p.H, y0 = lin - col * p.H, y1 = min(p.H, y0 + (lin1 - lin));
             const int n = col / p.strips, sx = col - n * p.strips;
+            int lx0 = 0, next_k = 0;             // up2: first source column of the strip, next half-resolution row to stage
+            if (UP2) {
+                int i1; float l0, l1;
+                up2_coord(sx * 256, uw2, up2_scale(uw2), lx0, i1, l0, l1);
+                up2_coord(y0, uh2, up2_scale(uh2), next_k, i1, l0, l1);
+            }
+            // everything the epilogue reads for output row y of this segment
+            auto stage_operands = [&](int y) {
+                if constexpr (MASK || ADDS) {
+                    const uint32_t s = o % C::OPD;
+                    tc::mbar_wait(op_empty + 8 * s, ((o / C::OPD) & 1) ^ 1);
+                    if (elect_one()) {
+                        const uint32_t dst = op_s + s * C::NOPS * C::OP_BYTES;
+                        tc::mbar_arrive_expect_tx(op_full + 8 * s, C::NOPS * C::OP_BYTES);
+                        if (MASK) tc::tma_load_4d(dst, &tmap_mask, op_full + 8 * s, 0, sx * 128, y, n);
+                        if (ADDS) tc::tma_load_4d(dst + (MASK ? C::OP_BYTES : 0), &tmap_add, op_full + 8 * s, 0, sx * 128, y, n);
+                    }
+                    __syncwarp();
+                    ++o;
+                }
+                if constexpr (UP2) {
+                    int k0, k1; float l0, l1;
+                    up2_coord(y, uh2, up2_scale(uh2), k0, k1, l0, l1);
+                    for (; next_k <= k1; ++next_k, ++u) {
+                        const uint32_t s = u % C::UPD;
+                        tc::mbar_wait(up_empty + 8 * s, ((u / C::UPD) & 1) ^ 1);
+                        if (elect_one()) {
+                            tc::mbar_arrive_expect_tx(up_full + 8 * s, C::UP_BYTES);
+                            tc::tma_load_4d(up_s + s * C::UP_SLOT, &tmap_up, up_full + 8 * s, 0, lx0, next_k, n);
+                        }
+                        __syncwarp();
+                    }
+                }
+            };
             for (int yy = y0 - 1; yy <= y1; ++yy, ++r) {
                 const uint32_t slot = r % C::RB;
                 tc::mbar_wait(row_free + 8 * slot, ((r / C::RB) & 1) ^ 1);
                 if (elect_one()) {
                     tc::mbar_arrive_expect_tx(row_full + 8 * slot, C::ROW_BYTES);
                     tc::tma_load_4d(rows_s + slot * C::SLOT_BYTES, &tmap_in, row_full + 8 * slot, 0, sx * 128 - 1, yy, n);
-                    if (NC == 32 && yy >= y0 && yy < y1 && (p.mask || p.add || p.add2)) {       // the epilogue reads these rows ~3 input rows from now
-                        const size_t roff = (((size_t)n * p.H + yy) * p.W + sx * 256) * 32;
-                        const uint32_t rbytes = (uint32_t)min(256, p.W - sx * 256) * 64u;
-                        if (p.mask) tc::l2_prefetch(p.mask + roff, rbytes);
-                        if (p.add) tc::l2_prefetch(p.add + roff, rbytes);
-                        if (p.add2) tc::l2_prefetch(p.add2 + roff, rbytes);
-                    }
                 }
                 __syncwarp();
+                if ((MASK || ADDS || UP2) && yy - C::LAG >= y0) stage_operands(yy - C::LAG);
             }
+            if (MASK || ADDS || UP2)
+                for (int y = max(y0, y1 + 1 - C::LAG); y < y1; ++y) stage_operands(y);
             lin += y1 - y0;
         }
     } else if (warp == 1) {
@@ -409,8 +448,7 @@ __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, cons
         float bias[32];
 #pragma unroll
         for (int c = 0; c < 32; ++c) bias[c] = p.bias ? __ldg(p.bias + c) : 0.f;
-        const bf16* addsrc = ADDS ? (p.add ? p.add : p.add2) : nullptr;     // the two are never used together
-        uint32_t t = 0;
+        uint32_t t = 0, ubase = 0;               // output rows done, half-resolution rows of earlier segments
         for (int lin = lin0; lin < lin1;) {
             const int col = lin / p.H, y0 = lin - col * p.H, y1 = min(p.H, y0 + (lin1 - lin));
             const int n = col / p.strips, sx = col - n * p.strips;
@@ -418,27 +456,40 @@ __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, cons
             const int xw = sx * 256 + q * 64;                                // first pixel of this quarter
             const int vp = min(32, (p.W - xw) / 2);                          // valid pixel pairs of this quarter (may be <= 0)
             const bool act = lane < vp;
-            // bilinear x2 addend: this thread's column pair and weights are the same for every row of the segment
-            int ux0 = 0, ux1 = 0; float ulx0 = 0.f, ulx1 = 0.f;
-            const int uh2 = p.H >> 1, uw2 = p.W >> 1;
-            if (UP2 && act) up2_coord(xw + 2 * lane + par, uw2, up2_scale(uw2), ux0, ux1, ulx0, ulx1);
+            // bilinear x2 addend: this thread's column pair and weights are the same for every row of the segment; the staged
+            // half-resolution rows start at the strip's first source column lx0 and run k_lo .. k_hi
+            int ux0 = 0, ux1 = 0, lx0 = 0, k_lo = 0, k_hi = 0, rel = 0; float ulx0 = 0.f, ulx1 = 0.f;
+            if (UP2) {
+                int i1; float l0, l1;
+                up2_coord(sx * 256, uw2, up2_scale(uw2), lx0, i1, l0, l1);
+                up2_coord(y0, uh2, up2_scale(uh2), k_lo, i1, l0, l1);
+                up2_coord(y1 - 1, uh2, up2_scale(uh2), i1, k_hi, l0, l1);
+                rel = k_lo;
+                if (act) {
+                    up2_coord(xw + 2 * lane + par, uw2, up2_scale(uw2), ux0, ux1, ulx0, ulx1);
+                    ux0 -= lx0; ux1 -= lx0;
+                }
+            }
             for (int y = y0; y < y1; ++y, ++t) {
                 const uint32_t sl = t % C::NSLOT;
-                // this thread's pixel: 64 contiguous bytes of every NHWC map; mask / add are fetched BEFORE waiting for the accumulators
-                const size_t off = (((size_t)n * p.H + y) * p.W + xw + 2 * lane + par) * 32;
                 float up[32];
-                if (UP2) {
+                if constexpr (UP2) {
+                    int uy0, uy1; float uly0, uly1;
+                    up2_coord(y, uh2, up2_scale(uh2), uy0, uy1, uly0, uly1);
+                    const uint32_t g0 = ubase + (uint32_t)(uy0 - k_lo), g1 = ubase + (uint32_t)(uy1 - k_lo);
+                    tc::mbar_wait(up_full + 8 * (g0 % C::UPD), (g0 / C::UPD) & 1);
+                    tc::mbar_wait(up_full + 8 * (g1 % C::UPD), (g1 / C::UPD) & 1);
                     if (act) {
-                        int uy0, uy1; float uly0, uly1;
-                        up2_coord(y, uh2, up2_scale(uh2), uy0, uy1, uly0, uly1);
-                        const bf16* hb = p.up2 + (size_t)n * uh2 * uw2 * 32;
-                        const uint4* r00 = reinterpret_cast<const uint4*>(hb + ((size_t)uy0 * uw2 + ux0) * 32);
-                        const uint4* r01 = reinterpret_cast<const uint4*>(hb + ((size_t)uy0 * uw2 + ux1) * 32);
-                        const uint4* r10 = reinterpret_cast<const uint4*>(hb + ((size_t)uy1 * uw2 + ux0) * 32);
-                        const uint4* r11 = reinterpret_cast<const uint4*>(hb + ((size_t)uy1 * uw2 + ux1) * 32);
+                        // pixel x of a staged row: 64 B at x * 64, 16 B chunk g at ((g ^ ((x >> 1) & 3)) << 4) (SWIZZLE_64B)
+                        const unsigned char* hr0 = smem + (up_s - smem_base) + (g0 % C::UPD) * C::UP_SLOT;
+                        const unsigned char* hr1 = smem + (up_s - smem_base) + (g1 % C::UPD) * C::UP_SLOT;
+                        const int sw0 = (ux0 >> 1) & 3, sw1 = (ux1 >> 1) & 3;
 #pragma unroll
                         for (int g = 0; g < 4; ++g) {
-                            const uint4 a00 = __ldg(r00 + g), a01 = __ldg(r01 + g), a10 = __ldg(r10 + g), a11 = __ldg(r11 + g);
+                            const uint4 a00 = *reinterpret_cast<const uint4*>(hr0 + ux0 * 64 + ((g ^ sw0) << 4));
+                            const uint4 a01 = *reinterpret_cast<const uint4*>(hr0 + ux1 * 64 + ((g ^ sw1) << 4));
+                            const uint4 a10 = *reinterpret_cast<const uint4*>(hr1 + ux0 * 64 + ((g ^ sw0) << 4));
+                            const uint4 a11 = *reinterpret_cast<const uint4*>(hr1 + ux1 * 64 + ((g ^ sw1) << 4));
                             const uint32_t *u00 = reinterpret_cast<const uint32_t*>(&a00), *u01 = reinterpret_cast<const uint32_t*>(&a01);
                             const uint32_t *u10 = reinterpret_cast<const uint32_t*>(&a10), *u11 = reinterpret_cast<const uint32_t*>(&a11);
 #pragma unroll
@@ -452,13 +503,13 @@ __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, cons
 #pragma unroll
                         for (int c = 0; c < 32; ++c) up[c] = 0.f;
                     }
+                    // half-resolution rows no later output row of the segment reads go back to the producer
+                    int keep = k_hi + 1;
+                    if (y + 1 < y1) { int i1; float l0, l1; up2_coord(y + 1, uh2, up2_scale(uh2), keep, i1, l0, l1); }
+                    __syncwarp();
+                    for (; rel < keep; ++rel)
+                        if (lane == 0) tc::mbar_arrive(up_empty + 8 * ((ubase + (uint32_t)(rel - k_lo)) % C::UPD));
                 }
-                uint4 mk[4], ad[4];
-                OperandRows mrows, arows;
-                // first pixel of this warp's parity in the row: the loads below are issued BEFORE waiting for the accumulators
-                const size_t off_q = (((size_t)n * p.H + y) * p.W + xw + par) * 32;
-                if (MASK) operand_rows_load(mrows, p.mask + off_q, vp, lane, true);
-                if (ADDS) operand_rows_load(arows, addsrc + off_q, vp, lane, false);          // may alias `out`: plain loads
                 tc::mbar_wait(slot_full + 8 * sl, (t / C::NSLOT) & 1);
                 tc::tc_fence_after();
                 uint32_t v[32];
@@ -466,9 +517,21 @@ __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, cons
                 tc::tc_fence_before();
                 __syncwarp();
                 if (lane == 0) tc::mbar_arrive(slot_empty + 8 * sl);
+                uint4 mk[4], ad[4];
+                if constexpr (MASK || ADDS) {            // this pixel's 64 B of the staged rows: where its output goes in the staging tile
+                    const uint32_t os = t % C::OPD;
+                    tc::mbar_wait(op_full + 8 * os, (t / C::OPD) & 1);
+                    const unsigned char* orow = smem + (op_s - smem_base) + os * C::NOPS * C::OP_BYTES + (q * 32 + lane) * 128;
+#pragma unroll
+                    for (int g = 0; g < 4; ++g) {
+                        const int ch = ((par * 4 + g) ^ (lane & 7)) << 4;
+                        if (MASK) mk[g] = *reinterpret_cast<const uint4*>(orow + ch);
+                        if (ADDS) ad[g] = *reinterpret_cast<const uint4*>(orow + (MASK ? C::OP_BYTES : 0) + ch);
+                    }
+                    __syncwarp();
+                    if (lane == 0) tc::mbar_arrive(op_empty + 8 * os);
+                }
                 if (vp <= 0) continue;                   // whole quarter right of the image: both of its warps skip
-                if (MASK) operand_rows_transpose(mrows, lane, mk);
-                if (ADDS) operand_rows_transpose(arows, lane, ad);
                 uint4 ov[4], ov_pre[4];
                 conv_tc_pixel(v, bias, MASK ? mk : nullptr, (ADDS && p.add) ? ad : nullptr, p.relu_out, ov, UP2 ? up : nullptr,
                               (p.out2 && p.out2_pre_add) ? ov_pre : nullptr);
@@ -476,7 +539,7 @@ __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, cons
                 unsigned char* srow = smem + (stage_q - smem_base) + buf + lane * 128;
 #pragma unroll
                 for (int g = 0; g < 4; ++g) *reinterpret_cast<uint4*>(srow + (((par * 4 + g) ^ (lane & 7)) << 4)) = ov[g];
-                if (p.out2) {                            // out2 = ReLU(bf16(out) [+ add2])
+                if (C::OUT2 && p.out2) {                 // out2 = ReLU(bf16(out) [+ add2])
                     unsigned char* srow2 = srow + C::STAGE_BYTES;
 #pragma unroll
                     for (int g = 0; g < 4; ++g) {
@@ -503,10 +566,11 @@ __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, cons
                 tc::named_bar_sync(1 + q, 64);           // both warps of the quarter have written their halves of the pair rows
                 if (issuer) {
                     tc::tma_store_4d(&tmap_out, stage_q + buf, 0, xw >> 1, y, n);
-                    if (p.out2) tc::tma_store_4d(&tmap_out2, stage2_q + buf, 0, xw >> 1, y, n);
+                    if (C::OUT2 && p.out2) tc::tma_store_4d(&tmap_out2, stage2_q + buf, 0, xw >> 1, y, n);
                     tc::bulk_store_commit();
                 }
             }
+            if (UP2) ubase += (uint32_t)(k_hi - k_lo + 1);
         }
         if (issuer) tc::bulk_store_wait_read_all();      // shared memory may go once the stores have READ it; the grid's completion
                                                          // makes the writes visible (what CUTLASS's tma_store_wait does)
@@ -521,19 +585,24 @@ __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, cons
     }
 }
 
+// tmap_mask / tmap_add: the mask and the add (or add2) map in the pair-row view with 128-pair boxes; tmap_up: the half-resolution
+// map with UP_BOX-pixel boxes (each only read by the instantiation that uses it)
 template <bool MASK, bool ADDS, bool UP2>
-__global__ void __launch_bounds__(ConvTcCfg::THREADS, 1) conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap_in,
-                                                                           const __grid_constant__ CUtensorMap tmap_out,
-                                                                           const __grid_constant__ CUtensorMap tmap_out2, const ConvTcParams p) {
-    conv3x3_tc_body<32, MASK, ADDS, UP2>(tmap_in, tmap_out, tmap_out2, p);
+__global__ void __launch_bounds__(ConvTcCfg<>::THREADS, 1) conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap_in,
+                                                                             const __grid_constant__ CUtensorMap tmap_out,
+                                                                             const __grid_constant__ CUtensorMap tmap_out2,
+                                                                             const __grid_constant__ CUtensorMap tmap_mask,
+                                                                             const __grid_constant__ CUtensorMap tmap_add,
+                                                                             const __grid_constant__ CUtensorMap tmap_up, const ConvTcParams p) {
+    conv3x3_tc_body<32, MASK, ADDS, UP2>(tmap_in, tmap_out, tmap_out2, tmap_mask, tmap_add, tmap_up, p);
 }
 
 // 32 -> 1 channel 3x3 s1 p1 convolution with an fp32 output plane: the prediction layer prdct.3 (network_exp_msg_chn_adapt.py:289)
 // and, with flipped plane-1 weights, the data gradient of a two-plane stem with respect to its prediction input.  The layer reads
 // 64 B and writes 4 B per pixel: it is bound by the read of the 32-channel map, which the tensor-core form streams through TMA exactly
 // once (the CUDA-core form staged halo tiles and spent 288 shared-memory-fed FMAs per pixel: 22 us at 352x1216).
-__global__ void __launch_bounds__(ConvTcCfg::THREADS, 1) conv3x3_tc_head_kernel(const __grid_constant__ CUtensorMap tmap_in, const ConvTcParams p) {
-    conv3x3_tc_body<16, false, false, false>(tmap_in, tmap_in, tmap_in, p);
+__global__ void __launch_bounds__(ConvTcCfg<>::THREADS, 1) conv3x3_tc_head_kernel(const __grid_constant__ CUtensorMap tmap_in, const ConvTcParams p) {
+    conv3x3_tc_body<16, false, false, false>(tmap_in, tmap_in, tmap_in, tmap_in, tmap_in, tmap_in, p);
 }
 
 // fp32 [tap][cin] (tap = ky*3 + kx) -> the head kernel's weight image: row = kx*48 + (2-ky)*16 + c, 64 B per row (32 cin), SWIZZLE_64B
@@ -577,7 +646,7 @@ inline int make_tmap_nhwc(CUtensorMap* map, const void* ptr, int N, int H, int W
 }
 
 // NHWC bf16 [N,H,W,32] activation viewed as [N][H][W/2][64]: box = {64, 130 pairs, 1, 1}, SWIZZLE_128B, zero fill outside
-inline int make_tmap_pairs(CUtensorMap* map, const void* ptr, int N, int H, int W, int box_pairs = ConvTcCfg::BOXP) {
+inline int make_tmap_pairs(CUtensorMap* map, const void* ptr, int N, int H, int W, int box_pairs = ConvTcCfg<>::BOXP) {
     PFN_encodeTiled enc = get_encode_tiled();
     PTTA_CHECK(enc != nullptr, "cuTensorMapEncodeTiled not available from the driver");
     cuuint64_t dims[4] = {64, (cuuint64_t)(W / 2), (cuuint64_t)H, (cuuint64_t)N};
@@ -593,16 +662,18 @@ inline int make_tmap_pairs(CUtensorMap* map, const void* ptr, int N, int H, int 
 
 inline bool conv_tc_supported(int N, int H, int W) { return N >= 1 && H >= 1 && W >= 2 && (W % 2) == 0; }
 
-// tensor maps are cached per (pointer, shape): the engine's arena addresses are fixed, so a step encodes nothing
-inline int conv_tc_tmap(const bf16* in, int N, int H, int W, const CUtensorMap** out, int box_pairs = ConvTcCfg::BOXP) {
-    struct Entry { const void* ptr; int n, h, w, box; CUtensorMap map; };
+// tensor maps are cached per (pointer, shape, box): the engine's arena addresses are fixed, so a step encodes nothing.
+// pairs = true: the [N][H][W/2][64] pair-row view with `box` pairs per box; false: the plain NHWC view with `box` pixels (SWIZZLE_64B)
+inline int conv_tc_tmap(const bf16* in, int N, int H, int W, const CUtensorMap** out, int box = ConvTcCfg<>::BOXP, bool pairs = true) {
+    struct Entry { const void* ptr; int n, h, w, box; bool pairs; CUtensorMap map; };
     static thread_local std::vector<Entry> cache;
     for (const Entry& e : cache)
-        if (e.ptr == in && e.n == N && e.h == H && e.w == W && e.box == box_pairs) { *out = &e.map; return 0; }
+        if (e.ptr == in && e.n == N && e.h == H && e.w == W && e.box == box && e.pairs == pairs) { *out = &e.map; return 0; }
     if (cache.size() >= 1024) cache.clear();
     cache.reserve(1024);              // pointers into the cache are handed out: never reallocate
-    Entry e; e.ptr = in; e.n = N; e.h = H; e.w = W; e.box = box_pairs;
-    PTTA_TRY(make_tmap_pairs(&e.map, in, N, H, W, box_pairs));
+    Entry e; e.ptr = in; e.n = N; e.h = H; e.w = W; e.box = box; e.pairs = pairs;
+    if (pairs) PTTA_TRY(make_tmap_pairs(&e.map, in, N, H, W, box));
+    else PTTA_TRY(make_tmap_nhwc(&e.map, in, N, H, W, 32, box));
     cache.push_back(e);
     *out = &cache.back().map;
     return 0;
@@ -627,7 +698,7 @@ inline int conv_tc_split(ConvTcParams& p, int sms) {
 
 // out_f32[n][y][x] = bias0 [+ add_f32[n][y][x]] + sum_taps in[n][y+ky-1][x+kx-1][:] . w[tap][:]   (p.w = image of pack_conv_weight_tc_head_kernel)
 inline int launch_conv_tc_head(const bf16* in, ConvTcParams p, cudaStream_t st) {
-    typedef ConvTcCfg C;
+    typedef ConvTcCfg<> C;
     static int sms = 0;
     if (!sms) {
         PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_head_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
@@ -645,22 +716,30 @@ inline int launch_conv_tc_head(const bf16* in, ConvTcParams p, cudaStream_t st) 
     return check_launch("conv3x3_tc_head");
 }
 
+template <bool MASK, bool ADDS, bool UP2>
+inline void launch_conv_tc_variant(int grid, cudaStream_t st, const CUtensorMap& map_in, const CUtensorMap& map_out, const CUtensorMap& map_out2,
+                                   const CUtensorMap& map_mask, const CUtensorMap& map_add, const CUtensorMap& map_up, const ConvTcParams& p) {
+    typedef ConvTcCfg<MASK, ADDS, UP2> C;
+    launch_k(conv3x3_tc_kernel<MASK, ADDS, UP2>, grid, C::THREADS, C::SMEM, st, map_in, map_out, map_out2, map_mask, map_add, map_up, p);
+}
+
 inline int launch_conv_tc(const bf16* in, ConvTcParams p, cudaStream_t st) {
-    typedef ConvTcCfg C;
     static int sms = 0;
     if (!sms) {
-        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
-        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
-        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
-        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
-        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
-        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
+        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ConvTcCfg<false, false, false>::SMEM));
+        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ConvTcCfg<false, true, false>::SMEM));
+        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ConvTcCfg<true, false, false>::SMEM));
+        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ConvTcCfg<true, true, false>::SMEM));
+        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ConvTcCfg<false, false, true>::SMEM));
+        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ConvTcCfg<false, true, true>::SMEM));
         int dev = 0;
         PTTA_CUDA(cudaGetDevice(&dev));
         PTTA_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     }
     PTTA_CHECK(conv_tc_supported(p.N, p.H, p.W), "conv3x3_tc: W=%d must be even", p.W);
     PTTA_CHECK(!(p.up2 && p.mask), "conv3x3_tc: the upsampled addend and a derivative mask are never used together");
+    PTTA_CHECK(!(p.out2 && p.mask), "conv3x3_tc: a derivative mask and the second output are never used together");
+    PTTA_CHECK(!(p.add && p.add2), "conv3x3_tc: add and add2 are mutually exclusive");
     PTTA_CHECK(!p.relu_in, "conv3x3_tc: ReLU-on-load is not supported (producers store ReLU(x): relu_out)");
     PTTA_CHECK(!p.up2 || ((p.H & 1) == 0 && (p.W & 1) == 0), "conv3x3_tc: the x2-upsampled addend needs even H, W (got %dx%d)", p.H, p.W);
     const int grid = conv_tc_split(p, sms);
@@ -670,18 +749,23 @@ inline int launch_conv_tc(const bf16* in, ConvTcParams p, cudaStream_t st) {
     const CUtensorMap map_in = *m;
     PTTA_TRY(conv_tc_tmap(p.out, p.N, p.H, p.W, &m, 32));
     const CUtensorMap map_out = *m;
-    CUtensorMap map_out2 = map_out;
+    CUtensorMap map_out2 = map_out, map_mask = map_out, map_add = map_out, map_up = map_out;
     if (p.out2) { PTTA_TRY(conv_tc_tmap(p.out2, p.N, p.H, p.W, &m, 32)); map_out2 = *m; }
-    const bool mask = p.mask != nullptr, adds = p.add != nullptr || p.add2 != nullptr, up2 = p.up2 != nullptr;
+    const bf16* addsrc = p.add ? p.add : p.add2;
+    const int opbox = ConvTcCfg<true>::OP_BYTES / 128;
+    if (p.mask) { PTTA_TRY(conv_tc_tmap(p.mask, p.N, p.H, p.W, &m, opbox)); map_mask = *m; }
+    if (addsrc) { PTTA_TRY(conv_tc_tmap(addsrc, p.N, p.H, p.W, &m, opbox)); map_add = *m; }
+    if (p.up2) { PTTA_TRY(conv_tc_tmap(p.up2, p.N, p.H / 2, p.W / 2, &m, ConvTcCfg<false, false, true>::UP_BOX, false)); map_up = *m; }
+    const bool mask = p.mask != nullptr, adds = addsrc != nullptr, up2 = p.up2 != nullptr;
     if (up2) {
-        if (adds) launch_k(conv3x3_tc_kernel<false, true, true>, grid, C::THREADS, C::SMEM, st, map_in, map_out, map_out2, p);
-        else launch_k(conv3x3_tc_kernel<false, false, true>, grid, C::THREADS, C::SMEM, st, map_in, map_out, map_out2, p);
+        if (adds) launch_conv_tc_variant<false, true, true>(grid, st, map_in, map_out, map_out2, map_mask, map_add, map_up, p);
+        else launch_conv_tc_variant<false, false, true>(grid, st, map_in, map_out, map_out2, map_mask, map_add, map_up, p);
     } else if (mask) {
-        if (adds) launch_k(conv3x3_tc_kernel<true, true, false>, grid, C::THREADS, C::SMEM, st, map_in, map_out, map_out2, p);
-        else launch_k(conv3x3_tc_kernel<true, false, false>, grid, C::THREADS, C::SMEM, st, map_in, map_out, map_out2, p);
+        if (adds) launch_conv_tc_variant<true, true, false>(grid, st, map_in, map_out, map_out2, map_mask, map_add, map_up, p);
+        else launch_conv_tc_variant<true, false, false>(grid, st, map_in, map_out, map_out2, map_mask, map_add, map_up, p);
     } else {
-        if (adds) launch_k(conv3x3_tc_kernel<false, true, false>, grid, C::THREADS, C::SMEM, st, map_in, map_out, map_out2, p);
-        else launch_k(conv3x3_tc_kernel<false, false, false>, grid, C::THREADS, C::SMEM, st, map_in, map_out, map_out2, p);
+        if (adds) launch_conv_tc_variant<false, true, false>(grid, st, map_in, map_out, map_out2, map_mask, map_add, map_up, p);
+        else launch_conv_tc_variant<false, false, false>(grid, st, map_in, map_out, map_out2, map_mask, map_add, map_up, p);
     }
     return check_launch("conv3x3_tc");
 }

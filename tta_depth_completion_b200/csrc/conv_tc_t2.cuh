@@ -25,8 +25,11 @@
 
 namespace ptta {
 
+// OPS: the instantiation that reads mask / add.  It gives up four input-row slots (still eight output rows of look-ahead: an input
+// row feeds two output rows) for one staging tile per epilogue warp and operand.
+template <bool OPS = false>
 struct ConvTcT2Cfg {
-    static const int RB = 8;                      // input-row slots in the shared-memory ring
+    static const int RB = OPS ? 4 : 8;            // input-row slots in the shared-memory ring
     static const int NSLOT = 4;                   // output-row accumulator slots per bank
     static const int BOXP = 130;                  // pixel pairs per staged row (the stride-1 kernel's tensor map; 129 are used)
     static const int ROW_BYTES = BOXP * 128;
@@ -34,9 +37,12 @@ struct ConvTcT2Cfg {
     static const int W_BYTES = 9 * 32 * 64;
     static const int OUT_TILE = 8192;             // one TMEM lane quarter's output row: 64 output pixel pairs x 128 B (one TMA store box)
     static const int STAGE_BYTES = 4 * 2 * OUT_TILE;   // 4 quarters x double buffer
+    static const int OP_TILE = 32 * 128;          // one epilogue warp's share of an output row of one operand: 32 lanes x 2 pixels x 64 B
+    static const int OP_BYTES = OPS ? 8 * 2 * OP_TILE : 0;     // [warp][mask | add]
     static const int BAR_BYTES = 1024;
-    static const int SMEM = 1024 + RB * SLOT_BYTES + W_BYTES + STAGE_BYTES + BAR_BYTES;
+    static const int SMEM = 1024 + RB * SLOT_BYTES + W_BYTES + STAGE_BYTES + OP_BYTES + BAR_BYTES;
     static const int THREADS = 320;               // warp 0 TMA producer | warp 1 MMA issuer | warps 2-9 epilogue
+    static_assert(SMEM <= 232448, "conv3x3_tc_t2: shared memory over the 227 KB a block can opt into");
 };
 
 // [tap][cout][cin] bf16 (tap = ky*3 + kx of the ConvTranspose2d weight as the mma.sync MODE_T2 kernel reads it) -> the kernel's
@@ -53,16 +59,22 @@ __global__ void pack_conv_weight_tc_t2_kernel(const bf16* __restrict__ pack, bf1
 }
 
 // p.H, p.W: INPUT size (W even); output 2H x 2W.  p.rows_per_cta / p.total_rows count INPUT rows.
-__global__ void __launch_bounds__(ConvTcT2Cfg::THREADS, 1) conv3x3_tc_t2_kernel(const __grid_constant__ CUtensorMap tmap_in,
-                                                                                const __grid_constant__ CUtensorMap tmap_out, const ConvTcParams p) {
-    typedef ConvTcT2Cfg C;
+// The thread's two output pixels are 128 contiguous bytes of every output-shaped map, at a 256 B stride between lanes.  Loaded by
+// the thread itself, every request of a mask / add row touches 32 lines; instead the warp copies its 32 x 128 B of each operand row
+// with cp.async, eight lanes per 128 B (4 lines per request), into a tile swizzled by lane (chunk c of lane l at
+// l * 128 + ((c ^ (l & 7)) << 4)), issued before the accumulator wait, and each thread reads its own 128 B back.
+template <bool OPS>
+__global__ void __launch_bounds__(ConvTcT2Cfg<>::THREADS, 1) conv3x3_tc_t2_kernel(const __grid_constant__ CUtensorMap tmap_in,
+                                                                                  const __grid_constant__ CUtensorMap tmap_out, const ConvTcParams p) {
+    typedef ConvTcT2Cfg<OPS> C;
     extern __shared__ unsigned char smem_raw[];
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     unsigned char* smem = smem_raw + (smem_base - smem_u32(smem_raw));
     const uint32_t rows_s = smem_base;
     const uint32_t w_s = smem_base + C::RB * C::SLOT_BYTES;
     const uint32_t stage_s = w_s + C::W_BYTES;
-    const uint32_t bar_s = stage_s + C::STAGE_BYTES;
+    const uint32_t op_s = stage_s + C::STAGE_BYTES;          // OPS: [epilogue warp][mask | add][OP_TILE]
+    const uint32_t bar_s = op_s + C::OP_BYTES;
     const uint32_t row_full = bar_s;                         // [RB]    TMA      -> MMA
     const uint32_t row_free = bar_s + 8 * C::RB;             // [RB]    MMA      -> producer
     const uint32_t slot_full = bar_s + 16 * C::RB;           // [NSLOT] MMA      -> epilogue
@@ -117,15 +129,6 @@ __global__ void __launch_bounds__(ConvTcT2Cfg::THREADS, 1) conv3x3_tc_t2_kernel(
                 if (elect_one()) {
                     tc::mbar_arrive_expect_tx(row_full + 8 * slot, C::ROW_BYTES);
                     tc::tma_load_4d(rows_s + slot * C::SLOT_BYTES, &tmap_in, row_full + 8 * slot, 0, sx * 128, yy, n);
-                    if (yy < y1 && (p.mask || p.add)) {            // output rows 2yy, 2yy+1 of this strip: read by the epilogue a few rows from now
-#pragma unroll
-                        for (int e = 0; e < 2; ++e) {
-                            const size_t roff = (((size_t)n * Ho + 2 * yy + e) * Wo + sx * 512) * 32;
-                            const uint32_t rbytes = (uint32_t)min(512, Wo - sx * 512) * 64u;
-                            if (p.mask) tc::l2_prefetch(p.mask + roff, rbytes);
-                            if (p.add) tc::l2_prefetch(p.add + roff, rbytes);
-                        }
-                    }
                 }
                 __syncwarp();
             }
@@ -193,6 +196,9 @@ __global__ void __launch_bounds__(ConvTcT2Cfg::THREADS, 1) conv3x3_tc_t2_kernel(
         const int half = (warp - 2) >> 2;                // 0: output pixels 4j, 4j+1 (banks 0, 1) | 1: 4j+2, 4j+3 (banks 2, 3)
         const bool issuer = half == 0 && lane == 0;
         const uint32_t stage_q = stage_s + q * 2 * C::OUT_TILE;
+        const uint32_t mst = op_s + (warp - 2) * 2 * C::OP_TILE, ast = mst + C::OP_TILE;   // this warp's operand tiles
+        const unsigned char* mrow = smem + (mst - smem_base) + lane * 128;
+        const unsigned char* arow = smem + (ast - smem_base) + lane * 128;
         tc::named_bar_sync(5, 256);                      // bias_sm written (epilogue warps only)
         uint32_t t = 0;
         for (int lin = lin0; lin < lin1;) {
@@ -201,22 +207,28 @@ __global__ void __launch_bounds__(ConvTcT2Cfg::THREADS, 1) conv3x3_tc_t2_kernel(
             lin += y1 - y0;
             const int jp = sx * 128 + q * 32;                                // first input pixel pair of this quarter
             const int vp = min(32, p.W / 2 - jp);                            // valid input pairs (may be <= 0)
-            const bool act = lane < vp;
             for (int R = 2 * y0; R < 2 * y1; ++R, ++t) {
                 const uint32_t sl = t % C::NSLOT;
-                // this thread's two output pixels: 128 contiguous bytes of every output-shaped NHWC map
-                const size_t off = (((size_t)n * Ho + R) * Wo + 4 * (jp + lane) + 2 * half) * 32;
-                uint4 mk[8], ad[8];
-                if (p.mask) {
+                if (OPS) {
+                    __syncwarp();                        // every lane has read the previous row's tiles
+                    // request k: lanes 8k'..8k'+7 copy the 128 B of lane s = 4k + (l >> 3), chunk l & 7; `add` may alias `out`: it is
+                    // read here, before this CTA's store of the row
 #pragma unroll
-                    for (int g = 0; g < 8; ++g) mk[g] = act ? __ldg(reinterpret_cast<const uint4*>(p.mask + off) + g) : make_uint4(0, 0, 0, 0);
-                }
-                if (p.add) {
-#pragma unroll
-                    for (int g = 0; g < 8; ++g) ad[g] = act ? *(reinterpret_cast<const uint4*>(p.add + off) + g) : make_uint4(0, 0, 0, 0);   // may alias `out`
+                    for (int k = 0; k < 8; ++k) {
+                        const int s = 4 * k + (lane >> 3), c = lane & 7;
+                        const size_t off = (((size_t)n * Ho + R) * Wo + 4 * (jp + s) + 2 * half) * 32 + c * 8;
+                        const uint32_t dst = s * 128 + ((c ^ (s & 7)) << 4);
+                        if (p.mask) cp_async16(mst + dst, p.mask + off, s < vp);
+                        if (p.add) cp_async16(ast + dst, p.add + off, s < vp);
+                    }
+                    cp_async_commit();
                 }
                 tc::mbar_wait(slot_full + 8 * sl, (t / C::NSLOT) & 1);
                 tc::tc_fence_after();
+                if (OPS) {
+                    cp_async_wait_all();
+                    __syncwarp();
+                }
                 const uint32_t buf = (t & 1) * C::OUT_TILE;
                 unsigned char* srow = smem + (stage_q - smem_base) + buf + (2 * lane + half) * 128;
                 const int swz = (2 * lane + half) & 7;
@@ -232,18 +244,19 @@ __global__ void __launch_bounds__(ConvTcT2Cfg::THREADS, 1) conv3x3_tc_t2_kernel(
                     float f[32];
 #pragma unroll
                     for (int c = 0; c < 32; ++c) f[c] = __uint_as_float(v[c]) + bias_sm[c];
-                    if (p.mask) {
+                    if (OPS && p.mask) {
 #pragma unroll
                         for (int g = 0; g < 4; ++g) {
-                            const uint32_t bits = positive_bits(mk[e * 4 + g]);
+                            const uint32_t bits = positive_bits(*reinterpret_cast<const uint4*>(mrow + (((e * 4 + g) ^ (lane & 7)) << 4)));
 #pragma unroll
                             for (int j = 0; j < 8; ++j) f[g * 8 + j] = (bits >> j) & 1u ? f[g * 8 + j] : 0.f;
                         }
                     }
-                    if (p.add) {
+                    if (OPS && p.add) {
 #pragma unroll
                         for (int g = 0; g < 4; ++g) {
-                            const uint32_t* au = reinterpret_cast<const uint32_t*>(&ad[e * 4 + g]);
+                            const uint4 av = *reinterpret_cast<const uint4*>(arow + (((e * 4 + g) ^ (lane & 7)) << 4));
+                            const uint32_t* au = reinterpret_cast<const uint32_t*>(&av);
 #pragma unroll
                             for (int j = 0; j < 4; ++j) {
                                 const float2 a = unpack_bf162(au[j]);
@@ -292,10 +305,10 @@ inline bool conv_tc_t2_supported(int N, int H, int W) { return N >= 1 && H >= 1 
 
 // in: [N, H, W, 32]; p.out (and p.mask / p.add): [N, 2H, 2W, 32]; p.N / p.H / p.W describe the INPUT
 inline int launch_conv_tc_t2(const bf16* in, ConvTcParams p, cudaStream_t st) {
-    typedef ConvTcT2Cfg C;
     static int sms = 0;
     if (!sms) {
-        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_t2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
+        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_t2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ConvTcT2Cfg<false>::SMEM));
+        PTTA_CUDA(cudaFuncSetAttribute(conv3x3_tc_t2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ConvTcT2Cfg<true>::SMEM));
         int dev = 0;
         PTTA_CUDA(cudaGetDevice(&dev));
         PTTA_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
@@ -320,7 +333,8 @@ inline int launch_conv_tc_t2(const bf16* in, ConvTcParams p, cudaStream_t st) {
     const CUtensorMap map_in = *m;
     PTTA_TRY(conv_tc_tmap(p.out, p.N, 2 * p.H, 2 * p.W, &m, 64));
     const CUtensorMap map_out = *m;
-    launch_k(conv3x3_tc_t2_kernel, grid, C::THREADS, C::SMEM, st, map_in, map_out, p);
+    if (p.mask || p.add) launch_k(conv3x3_tc_t2_kernel<true>, grid, ConvTcT2Cfg<true>::THREADS, ConvTcT2Cfg<true>::SMEM, st, map_in, map_out, p);
+    else launch_k(conv3x3_tc_t2_kernel<false>, grid, ConvTcT2Cfg<false>::THREADS, ConvTcT2Cfg<false>::SMEM, st, map_in, map_out, p);
     return check_launch("conv3x3_tc_t2");
 }
 
