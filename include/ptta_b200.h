@@ -233,10 +233,6 @@ int ptta_convg_run_thin(const void* x0_bf16, const void* x1_bf16, const void* pa
 int ptta_nl_stem(const float* image_nchw, const float* depth, const float* w_rgb, const float* b_rgb, const float* w_dep,
                  const float* b_dep, const float* scale3, const float* shift3, void* out_bf16_c64, int n, int h, int w,
                  ptta_stream_t stream);
-/* merged batch: out [2n,h,w,64] = the n real images followed by their zero-image copies (same sparse depth), one launch */
-int ptta_nl_stem_pair(const float* image_nchw, const float* depth, const float* w_rgb, const float* b_rgb, const float* w_dep,
-                      const float* b_dep, const float* scale3, const float* shift3, void* out_bf16_c64, int n, int h, int w,
-                      ptta_stream_t stream);
 /* number of partial blocks the reductions below use: `partial` must hold 2 * c * blocks floats */
 int ptta_nl_reduce_blocks(long long rows, int c);
 /* train-mode BatchNorm statistics (batch mean, biased variance) -> mean, rstd, scale = gamma*rstd, shift = beta - mean*scale;
@@ -244,15 +240,6 @@ int ptta_nl_reduce_blocks(long long rows, int c);
 int ptta_nl_bn_stats(const void* x_bf16, long long ldx, long long rows, int c, const float* gamma, const float* beta, float eps,
                      float* partial, float* mean, float* rstd, float* scale, float* shift, float* run_mean, float* run_var,
                      long long* num_batches_tracked, float momentum, ptta_stream_t stream);
-/* the same statistics for `groups` independent row ranges of rows_per_group rows each (real | zero-image halves of a merged
- * batch: each half is its own forward pass in the reference, nlspnmodel_adapt.py:866-914); outputs are [groups][c]; `partial` must
- * hold groups * 2 * c * ptta_nl_reduce_blocks(rows_per_group, c) floats.  ptta_nl_bn_act_grouped applies group g's vectors to its rows */
-int ptta_nl_bn_stats_grouped(const void* x_bf16, long long ldx, long long rows_per_group, int groups, int c, const float* gamma,
-                             const float* beta, float eps, float* partial, float* mean, float* rstd, float* scale, float* shift,
-                             ptta_stream_t stream);
-int ptta_nl_bn_act_grouped(const void* x_bf16, const float* scale, const float* shift, const void* res_bf16, long long ldr,
-                           const float* rscale, const float* rshift, void* y_bf16, long long rows_per_group, int groups, int c, int act,
-                           ptta_stream_t stream);
 int ptta_nl_col_sums(const void* x_bf16, long long ldx, long long rows, int c, float* partial, float* sums, ptta_stream_t stream);
 /* y = act(x*scale + shift [+ res | + res*rscale + rshift]); act: 0 none, 1 ReLU, 2 LeakyReLU(0.2) */
 int ptta_nl_bn_act(const void* x_bf16, const float* scale, const float* shift, const void* res_bf16, long long ldr,
@@ -371,7 +358,7 @@ void ptta_msgchn_destroy(ptta_msgchn* e);
 /* dispatch options (results stay right for every value; used by the parity tests to run ALL kernel families at every size):
  * "tc_min_pixels" / "tc_s2_min_pixels" / "tc_t2_min_pixels": smallest map (N*H*W of the INPUT) the stride-1 / stride-2 /
  * transposed tcgen05 convs take (0 = always),
- * "tc_enabled" 0/1, "two_streams" 0/1, "fuse_dec_sums" 0/1; "trainable_head" / "skip_dec3": see the preparation steps below.
+ * "tc_enabled" 0/1, "two_streams" 0/1; "trainable_head" / "skip_dec3": see the preparation steps below.
  * Unknown names fail. */
 /* ---- shared-model mode (BASELINE.json configs[4]; the reference: DDP + SyncBatchNorm, src/msg_chn_model_adapt.py:480,555-556) ----
  * One communicator per rank: a device block mapped into every peer through CUDA IPC.  With a communicator set, the engine's

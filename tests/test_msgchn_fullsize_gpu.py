@@ -185,27 +185,3 @@ def test_fused_proj3_pred0_equals_two_gemms():
     assert e < 1e-2, e
     assert rel(outs[0][1]['loss_cos'], outs[1][1]['loss_cos']) < 1e-3
     assert outs[0][1]['loss_sparse_depth'] == outs[1][1]['loss_sparse_depth']          # nothing else moved
-
-
-@pytest.mark.parametrize('opt', ['fuse_up2', 'fuse_enc_sums'])
-def test_epilogue_fusions_equal_the_separate_passes(opt):
-    """x = conv(.) + up2(pre_x) and the decoder sums x + c written by the encoder's conv epilogues (one rounding) against the separate
-    add_up2 / dec_sums passes (two roundings): same prediction and losses up to that rounding, same step."""
-    mode, cap = 'meta_selfsup_seq_2layers_ema', 80.0
-    sd = O.get_checkpoint('kitti_2layers_a', mode)
-    image, sparse, _ = O.synthetic_frame(15, 0, 1, 128, 256, 'kitti')
-    res = []
-    for on in (1, 0):
-        opts = {opt: on, 'tc_min_pixels': 0, 'tc_s2_min_pixels': 0, 'tc_t2_min_pixels': 0}
-        if opt == 'fuse_enc_sums':
-            opts['fuse_up2'] = 1
-        model = make_model(mode, sd, cap, options=opts)
-        model.tta_step(image.to(DEV), sparse.to(DEV), 1e-4, W_SD, W_SM, W_COS)
-        eng = model._last_engine
-        res.append((model.last_output().cpu().clone(), model.last_losses(), eng.tensor('real.d3.x0').float().cpu().clone(),
-                    eng.tensor('real.e3.x1r').float().cpu().clone(), {k: v.detach().cpu().clone() for k, v in model.state_dict().items() if 'meta' in k}))
-    # one bf16 rounding (2^-9 = 2e-3 per value) more or less at every level of the two cascades
-    assert nrel(res[0][0], res[1][0]) < 5e-3
-    for k in ('loss', 'loss_sparse_depth', 'loss_smooth', 'loss_cos'):
-        assert rel(res[0][1][k], res[1][1][k]) < 3e-3, (k, res[0][1][k], res[1][1][k])
-    assert nrel(res[0][2], res[1][2]) < 5e-3 and nrel(res[0][3], res[1][3]) < 5e-3

@@ -359,28 +359,6 @@ def test_graph_replay_equals_eager():
         assert torch.equal(a.state_dict()[k], b.state_dict()[k]), k
 
 
-def test_fused_bn_finalize_option_is_bit_identical():
-    """engine option fuse_bn_finalize = 1 (BatchNorm finalize inside col_stats, last-ticket blocks) against the default separate launches:
-    same slices, same summation order -- losses, adapted tensors and BatchNorm buffers bit for bit over 3 steps, 10 launches fewer"""
-    mode, cap, lr = 'meta_selfsup_seq_2layers_ema', 80.0, 1e-4
-    sd = O.make_synthetic_checkpoint(0, mode)
-    a = make_model(mode, sd, cap)
-    b = make_model(mode, sd, cap, options={'fuse_bn_finalize': 1})
-    counts = []
-    for t in range(3):
-        image, sparse, _ = O.synthetic_frame(8, t, 2, 48, 80, 'kitti')
-        for m in (a, b):
-            l0 = m._last_engine.launch_count() if t else 0
-            m.tta_step(image.to(DEV), sparse.to(DEV), lr, W_SD, W_SM, W_COS)
-            if t:
-                counts.append(m._last_engine.launch_count() - l0)
-        assert a.last_losses() == b.last_losses(), t
-    sa, sb = a.state_dict(), b.state_dict()
-    for k in sa:
-        assert torch.equal(sa[k], sb[k]), k
-    assert counts[1] == counts[0] - 10, counts
-
-
 @pytest.mark.parametrize('ckpt', [0, 'kitti_2layers_a'], ids=['random', 'fitted'])
 def test_continual_adaptation_metrics_track_the_oracle(ckpt):
     """100 continual steps at 64x128 (the north-star criterion: MAE / RMSE within 0.5 % of the reference after adaptation).

@@ -1,17 +1,22 @@
 #!/usr/bin/env python
 """GPU experiment: in-situ kernel start times of a REPLAYED step graph (profiling build, python -m tta_depth_completion_b200.build stamps).
-Run with PTTA_B200_LIB=tta_depth_completion_b200/lib/libptta_b200_stamps.so [PTTA_ONE_STREAM=1].  Kernel names come from one eager
-trace of the same step (same launch order on a single stream)."""
+Run with PTTA_B200_LIB=tta_depth_completion_b200/lib/libptta_b200_stamps.so: python tools/graph_stamps.py [workload] [--one-stream].
+--one-stream sets the engine option two_streams = 0, so the replayed graph launches in the order of one eager trace of the same step,
+which gives the kernel names."""
 import sys, os, ctypes, io, contextlib, subprocess
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 import bench
 from tta_depth_completion_b200 import ExternalModel_Adapt, _lib
 dev = torch.device('cuda:0')
-wl = sys.argv[1] if len(sys.argv) > 1 else 'kitti'
+args = [a for a in sys.argv[1:] if a != '--one-stream']
+one_stream = '--one-stream' in sys.argv[1:]
+wl = args[0] if args else 'kitti'
 h, w, dataset, mode, lr, cap = bench.WORKLOADS[wl]
 model = ExternalModel_Adapt('msg_chn', 0.0, 100.0, max_input_depth=cap, device=dev)
 model._prepare_head(mode)
+if one_stream:
+    model.model.engine_options = {'two_streams': 0}
 model.load_state_dict(bench.make_checkpoint(wl))
 model.set_image_normalization((1 / 255.0,) * 3, (0.0,) * 3)
 model.train()
@@ -42,7 +47,6 @@ with torch.cuda.stream(st):
                                                  _lib.ptr(frames[0][1]), cap, 1.0, 1.0, 0.1, ctypes.c_void_p(st.cuda_stream)), 'trace_step')
 os.dup2(saved, 1); os.close(wfd)
 names = [l.split()[-1] for l in os.read(r, 1 << 20).decode().splitlines() if l.strip()]
-one_stream = bool(os.environ.get('PTTA_ONE_STREAM'))
 if one_stream and len(names) == n:
     agg = {}
     for i in range(n):
@@ -53,6 +57,6 @@ if one_stream and len(names) == n:
     for k, a in sorted(agg.items(), key=lambda kv: -kv[1][1]):
         print('%-22s %3d launches  %7.1f us  avg %5.1f' % (k, a[0], a[1], a[1] / a[0]))
 else:
-    print('(%d names vs %d stamps: per-kernel attribution needs PTTA_ONE_STREAM=1)' % (len(names), n))
+    print('(%d names vs %d stamps: per-kernel attribution needs --one-stream)' % (len(names), n))
     gaps = [(ts[i + 1] - ts[i]) / 1e3 for i in range(n - 1)]
     print('start-to-start gaps: median %.1f us, max %.1f us' % (sorted(gaps)[len(gaps) // 2], max(gaps)))

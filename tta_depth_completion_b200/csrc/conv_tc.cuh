@@ -25,8 +25,6 @@ struct ConvTcParams {
     int relu_out;        // store ReLU(result) (producer-side activation for consumers that only read ReLU(x))
     int strips, segs_y, rows_per_seg, total_segs;      // stride-2 kernel: fixed row segments per strip
     int rows_per_cta, total_rows;                      // stride-1 kernel: contiguous range of the (image, strip, row) sequence per CTA
-    int out2_pre_add;    // out2 = ReLU(conv + bias [+ up2]) taken BEFORE `add` joins `out` (an encoder level: out = x + rgb feature = the decoder's
-                         // sum, out2 = ReLU(x) = what the next stride-2 conv reads; x itself is never needed raw)
     const bf16* up2;     // optional: out = conv + bias + up2(half-resolution map [N][H/2][W/2][32]) (bilinear x2, align_corners = True): the
                          // cascade's `x = conv(.) + F.interpolate(pre_x)` (network_exp_msg_chn_adapt.py:172-186) without a pass of its own
     // 32 -> 1 channel form (conv3x3_tc_head_kernel): fp32 output plane, optional fp32 addend plane, scalar bias
@@ -155,22 +153,13 @@ __global__ void pack_conv_weight_tc_kernel(const bf16* __restrict__ pack, bf16* 
 // The producer stages output row y's operands after it issued input row y + LAG, so it can still run LAG rows ahead of the MMA.
 // Every mbarrier has one arrival per phase except slot_empty, op_empty and up_empty (one per epilogue warp).
 __device__ __forceinline__ void conv_tc_pixel(const uint32_t (&v)[32], const float (&bias)[32], const uint4* mk, const uint4* ad, int relu_out,
-                                              uint4 (&ov)[4], const float* up = nullptr, uint4* ov_pre = nullptr) {
+                                              uint4 (&ov)[4], const float* up = nullptr) {
     float f[32];
 #pragma unroll
     for (int c = 0; c < 32; ++c) f[c] = __uint_as_float(v[c]) + bias[c];
     if (up) {
 #pragma unroll
         for (int c = 0; c < 32; ++c) f[c] += up[c];
-    }
-    if (ov_pre) {                      // bf16 of the result before `add` (the caller applies the ReLU)
-#pragma unroll
-        for (int g = 0; g < 4; ++g) {
-            ov_pre[g].x = pack_bf162(f[g * 8 + 0], f[g * 8 + 1]);
-            ov_pre[g].y = pack_bf162(f[g * 8 + 2], f[g * 8 + 3]);
-            ov_pre[g].z = pack_bf162(f[g * 8 + 4], f[g * 8 + 5]);
-            ov_pre[g].w = pack_bf162(f[g * 8 + 6], f[g * 8 + 7]);
-        }
     }
     if (mk) {
 #pragma unroll
@@ -532,9 +521,8 @@ __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, cons
                     if (lane == 0) tc::mbar_arrive(op_empty + 8 * os);
                 }
                 if (vp <= 0) continue;                   // whole quarter right of the image: both of its warps skip
-                uint4 ov[4], ov_pre[4];
-                conv_tc_pixel(v, bias, MASK ? mk : nullptr, (ADDS && p.add) ? ad : nullptr, p.relu_out, ov, UP2 ? up : nullptr,
-                              (p.out2 && p.out2_pre_add) ? ov_pre : nullptr);
+                uint4 ov[4];
+                conv_tc_pixel(v, bias, MASK ? mk : nullptr, (ADDS && p.add) ? ad : nullptr, p.relu_out, ov, UP2 ? up : nullptr);
                 const uint32_t buf = (t & 1) * C::OUT_TILE;
                 unsigned char* srow = smem + (stage_q - smem_base) + buf + lane * 128;
 #pragma unroll
@@ -543,7 +531,7 @@ __device__ __forceinline__ void conv3x3_tc_body(const CUtensorMap& tmap_in, cons
                     unsigned char* srow2 = srow + C::STAGE_BYTES;
 #pragma unroll
                     for (int g = 0; g < 4; ++g) {
-                        uint4 val = p.out2_pre_add ? ov_pre[g] : ov[g];
+                        uint4 val = ov[g];
                         if (ADDS && p.add2) {
                             uint32_t* vu = reinterpret_cast<uint32_t*>(&val);
                             const uint32_t* au = reinterpret_cast<const uint32_t*>(&ad[g]);

@@ -132,8 +132,7 @@ struct LinearLayer {
 struct EncW { StemLayer init0; ConvLayer init2, e1a, e1b, e2a, e2b, e3a, e3b, e4a, e4b; int nenc = 2; };
 struct DecW { ConvLayer d2a, d2b, d1a, d1b, p1; HeadLayer p3; };
 
-struct EncAct { Map32 a0, x0, t1, x1, t2, x2; Map32 x0r, x1r;    // x0r / x1r = ReLU(x0) / ReLU(x1): inputs of the stride-2 convs
-                bool sum0_done = false, sum1_done = false; };      // the decoder's x0 / x1 sums were already written by this encoder's conv epilogues
+struct EncAct { Map32 a0, x0, t1, x1, t2, x2; Map32 x0r, x1r; };    // x0r / x1r = ReLU(x0) / ReLU(x1): inputs of the stride-2 convs
 struct DecAct { Map32 x2, x1, x0, u2, x3, s1, u1, x4, s0, h; Map32 x2r; Map1 out; };   // x2r = ReLU(x2): input of the transposed conv dec2.1
 struct Branch {
     Map32 c[5];            // rgb features (c[2] after the meta layer)
@@ -168,7 +167,6 @@ struct ptta_msgchn {
     bool two_streams = true;
     bool mlp_on_st3 = false;        // set by forward_impl for the duration of the real cascade
     bool tc_enabled = true; long long tc_min_pixels = 6000, tc_s2_min_pixels = 6000, tc_t2_min_pixels = 1500, tc_head_min_pixels = 20000, tc_stem_min_pixels = 20000;
-    bool fuse_dec_sums = true;      // experiment switches (environment: PTTA_NO_TC, PTTA_NO_FUSE_DEC_SUMS, PTTA_ONE_STREAM)
     Arena arena;
     size_t ws_bytes = 0;
     bool bound = false, packed = false;
@@ -185,14 +183,6 @@ struct ptta_msgchn {
     LinearLayer proj0, proj3, pred0, pred3;
     bf16* projpred_pack = nullptr; float* projpred_bias = nullptr;   // pred.0 o proj.3 as one Linear layer (zero-image rows: emb = pred(proj(z)))
     bool fuse_projpred = true;
-    bool fuse_enc_sums = false;      // decoder sums x0 + c0, x1 + c1 written by the encoder's conv epilogues (needs fuse_up2).  Measured 722 -> 733
-                                     // frames/s: the passes it removes (dec_sums 48 -> 11 us) come back as epilogue time of the tcgen05 conv, and the
-                                     // oracle's bf16 emulation does not round at its points -- off by default, kept as a tested option
-    bool fuse_bn_finalize = false;   // BatchNorm finalize inside col_stats (the blocks holding the last tickets finalise; single-GPU path): bit-identical
-                                     // to the separate bn_finalize / bn_bwd_finalize launches and 10 launches fewer per step, but MEASURED SLOWER
-                                     // (721 vs 731 frames/s): with programmatic dependent launch the finalize kernel's launch is already hidden, and the
-                                     // tail -- 16 blocks of 256 threads after every other block has finished -- costs more than it saves.  Tested option, off
-    bool fuse_up2 = true;            // x = conv(.) + up2(pre_x) in the epilogue of the tcgen05 conv (option fuse_up2 = 0: separate add_up2 pass)
     // shared-model mode (ptta_msgchn_set_comm): SyncBatchNorm sums and the gradient all-reduce go through peer memory (peer_comm.cuh)
     PeerComm comm;
     int next_xid = 0;                // exchange slots are handed out in call order; every rank runs the same sequence
@@ -479,12 +469,12 @@ struct ptta_msgchn {
         k0 = allocv<float>(512); k1 = allocv<float>(512); k2 = allocv<float>(512);
         long long max_rows = std::max<long long>(R, 1);
         partial_doubles = (size_t)cdiv(max_rows, STATS_ROWS_PER_BLOCK) * 2 * 512;
-        partial = allocv<double>(partial_doubles + 2);           // + the two counters of the fused finalize (StatsFin)
-        partial2 = allocv<double>(partial_doubles + 2);
+        partial = allocv<double>(partial_doubles);
+        partial2 = allocv<double>(partial_doubles);
         size_t wg = std::max(wgrad_partial_bytes(N, H / 4, W / 4, 32, 128), wgrad_partial_bytes(N, H / 4, W / 4, 128, 32));
         wgrad_ws = (float*)arena.take(wg);
         wgrad_ws2 = (float*)arena.take(wg);
-        partial3 = allocv<double>(partial_doubles + 2);
+        partial3 = allocv<double>(partial_doubles);
         losses = (LossScalars*)arena.take(sizeof(LossScalars));
         reg("losses", losses, 0, 5, 1, 1, 1);
         loss_map_blocks = std::min(cdiv((long long)H * W, LOSS_BLOCK * 4), 1184);
@@ -714,10 +704,10 @@ struct ptta_msgchn {
         return launch_conv_tc_t2(in.p, p, st);
     }
     int conv_tc(const bf16* image, const float* bias, const Map32& in, const Map32& out, int relu_out, const bf16* mask, const bf16* add,
-                bf16* out2 = nullptr, bool stride2 = false, const bf16* add2 = nullptr, const bf16* up2 = nullptr, int out2_pre_add = 0) {
+                bf16* out2 = nullptr, bool stride2 = false, const bf16* add2 = nullptr, const bf16* up2 = nullptr) {
         ConvTcParams p; memset(&p, 0, sizeof(p));
         p.w = image; p.bias = bias; p.out = out.p; p.out2 = out2; p.add2 = add2; p.mask = mask; p.add = add; p.N = in.n; p.H = in.h; p.W = in.w;
-        p.up2 = up2; p.out2_pre_add = out2_pre_add;
+        p.up2 = up2;
         p.relu_out = relu_out;
         return stride2 ? launch_conv_tc_s2(in.p, p, st) : launch_conv_tc(in.p, p, st);
     }
@@ -725,8 +715,8 @@ struct ptta_msgchn {
     // out2 (optional): a second copy holding ReLU(out), for outputs that are read both raw and through a tensor-core conv
     // add2 (with out2): out2 = ReLU(out + add2) -- the decoder sums s = ReLU(conv(..) + skip) without a separate pass
     // true when conv_fwd(L, in, ...) runs on the stride-1 tcgen05 kernel, whose epilogue can add a x2-upsampled half-resolution map
-    bool can_fuse_up2(const ConvLayer& L, const Map32& in) const {
-        return fuse_up2 && L.img_fwd && L.mode_fwd == MODE_S1 && use_tc(in) && (in.h & 1) == 0 && (in.w & 1) == 0;
+    bool up2_in_epilogue(const ConvLayer& L, const Map32& in) const {
+        return L.img_fwd && L.mode_fwd == MODE_S1 && use_tc(in) && (in.h & 1) == 0 && (in.w & 1) == 0;
     }
     int conv_fwd(const ConvLayer& L, const Map32& in, const Map32& out, int pro, const BnState* probn = nullptr, int relu_out = 0,
                  bf16* out2 = nullptr, const bf16* add2 = nullptr, const bf16* up2 = nullptr) {
@@ -872,15 +862,12 @@ struct ptta_msgchn {
         if (next_xid >= PTTA_COMM_MAX_XID) { set_error("shared-model mode: more than %d peer exchanges in one step", PTTA_COMM_MAX_XID); return -1; }
         return next_xid++;
     }
-    // fin: optional fused finalize (single-GPU path; its counters sit behind the partial buffer of the stream the call runs on)
-    int stats(const bf16* x, const bf16* dy, long long rows, int C, int mode, const BnState* s, int relu_mask, int& nblk, const StatsFin* fin = nullptr) {
+    int stats(const bf16* x, const bf16* dy, long long rows, int C, int mode, const BnState* s, int relu_mask, int& nblk) {
         nblk = cdiv(rows, STATS_ROWS_PER_BLOCK);
         PTTA_CHECK((size_t)nblk * 2 * C <= partial_doubles, "stats partial buffer too small");
-        StatsFin f; memset(&f, 0, sizeof(f));
-        if (fin) { f = *fin; f.counters = reinterpret_cast<unsigned int*>(partial + partial_doubles); }
         launch_k(col_stats_kernel, nblk, 256, 2 * 2048 * sizeof(double), st, x, dy, partial, rows, C, mode, s ? s->mean : nullptr,
                                                                       s ? s->invstd : nullptr, s ? s->scale : nullptr,
-                                                                      s ? s->shift : nullptr, relu_mask, f);
+                                                                      s ? s->shift : nullptr, relu_mask);
         return check_launch("col_stats");
     }
     // defer_running: compute the batch statistics now, leave the running-statistics update to bn_running_update (ordering)
@@ -890,11 +877,6 @@ struct ptta_msgchn {
         if (defer_running) { p.running_mean = nullptr; p.running_var = nullptr; p.num_batches_tracked = nullptr; }
         p.uvar = s.uvar;
         p.mean = s.mean; p.invstd = s.invstd; p.scale = s.scale; p.shift = s.shift; p.momentum = 0.1f; p.eps = 1e-5f;
-        if (training && comm.world == 1 && fuse_bn_finalize) {     // the last blocks of col_stats finalise: no second launch
-            StatsFin fin; memset(&fin, 0, sizeof(fin));
-            fin.kind = 1; fin.count = rows; fin.p = p;
-            return stats(x, nullptr, rows, L.c, 0, nullptr, 0, nblk, &fin);
-        }
         if (training) PTTA_TRY(stats(x, nullptr, rows, L.c, 0, nullptr, 0, nblk));
         const int xid = (training && comm.world > 1) ? take_xid() : 0;
         if (xid < 0) return 1;
@@ -913,14 +895,6 @@ struct ptta_msgchn {
     int bn_backward(const BnLayer& L, const BnState& s, const bf16* dy, const bf16* x, bf16* dx, long long rows, int relu_mask,
                     float* dgamma, float* dbeta) {
         int nblk = 0;
-        if (comm.world == 1 && fuse_bn_finalize) {
-            StatsFin fin; memset(&fin, 0, sizeof(fin));
-            fin.kind = 2; fin.count = rows; fin.gamma = L.gamma; fin.invstd = s.invstd; fin.dgamma = dgamma; fin.dbeta = dbeta;
-            fin.k0 = k0; fin.k1 = k1; fin.k2 = k2;
-            PTTA_TRY(stats(x, dy, rows, L.c, 1, &s, relu_mask, nblk, &fin));
-            launch_k(bn_bwd_apply_kernel, cdiv(rows, (256 / (L.c / 8)) * EW_ROWS), 256, 0, st, dy, x, dx, rows, L.c, s.mean, s.invstd, k0, k1, k2, s.scale, s.shift, relu_mask);
-            return check_launch("bn_bwd_apply");
-        }
         PTTA_TRY(stats(x, dy, rows, L.c, 1, &s, relu_mask, nblk));
         const int xid = comm.world > 1 ? take_xid() : 0;
         if (xid < 0) return 1;
@@ -964,44 +938,29 @@ struct ptta_msgchn {
         PTTA_TRY(bn_forward_stats(metaBn2, B.bn2, B.mg.p, rows, training, defer_running));
         return bn_apply(B.mg.p, B.c2raw.p, B.c[2].p, rows, 32, B.bn2, 0);
     }
-    // sum0 / sum1 (optional, with c0 / c1): the decoder that follows needs x0 + c0 and x1 + c1 (rgb features) and nothing else reads x0 / x1
-    // raw, so on the tcgen05 path the conv epilogue writes the SUM as its first output and ReLU(x) as its second (A.sum*_done tells
-    // run_decoder); otherwise x is stored raw and dec_sums adds later
     int run_encoder(const EncW& Wt, EncAct& A, const float* p0, const float* p1, const Map32* pre_x4, const Map32* pre_x3,
-                    const Map32* pre_x2, const Map32* sum0 = nullptr, const Map32* c0 = nullptr, const Map32* sum1 = nullptr,
-                    const Map32* c1 = nullptr) {
+                    const Map32* pre_x2) {
         const long long hw = (long long)A.a0.h * A.a0.w;
         PTTA_TRY(stem(Wt.init0, p0, hw, 1.f, 0.f, p1 ? p1 : p0, hw, 1.f, 0.f, p0, hw, 0.f, 0.f, A.a0));
         // a0, t1, t2 hold ReLU(.) (stored by their producers): the stride-1 convs need no prologue
         // x0 / x1 are needed through ReLU by the stride-2 convs (and as ReLU masks in backward): whoever writes them last also writes the ReLU copy
         // x_k = conv(.) + up2(pre_x): the upsampled addend rides in the epilogue of the tcgen05 conv (no pass of its own); maps too small
         // for that kernel keep the separate add_up2 pass
-        A.sum0_done = A.sum1_done = false;
-        if (pre_x4 && can_fuse_up2(Wt.init2, A.a0)) {
-            if (sum0 && fuse_enc_sums) {
-                PTTA_TRY(conv_tc(Wt.init2.img_fwd, Wt.init2.b, A.a0, *sum0, 0, nullptr, c0->p, A.x0r.p, false, nullptr, pre_x4->p, 1));
-                A.sum0_done = true;
-            } else {
-                PTTA_TRY(conv_fwd(Wt.init2, A.a0, A.x0, PRO_NONE, nullptr, 0, A.x0r.p, nullptr, pre_x4->p));
-            }
+        if (pre_x4 && up2_in_epilogue(Wt.init2, A.a0)) {
+            PTTA_TRY(conv_fwd(Wt.init2, A.a0, A.x0, PRO_NONE, nullptr, 0, A.x0r.p, nullptr, pre_x4->p));
         } else {
             PTTA_TRY(conv_fwd(Wt.init2, A.a0, A.x0, PRO_NONE, nullptr, 0, pre_x4 ? nullptr : A.x0r.p));
             if (pre_x4) PTTA_TRY(add_up2(A.x0, *pre_x4, A.x0r.p));
         }
         PTTA_TRY(conv_fwd(Wt.e1a, A.x0r, A.t1, PRO_NONE, nullptr, 1));
-        if (pre_x3 && can_fuse_up2(Wt.e1b, A.t1)) {
-            if (sum1 && fuse_enc_sums) {
-                PTTA_TRY(conv_tc(Wt.e1b.img_fwd, Wt.e1b.b, A.t1, *sum1, 0, nullptr, c1->p, A.x1r.p, false, nullptr, pre_x3->p, 1));
-                A.sum1_done = true;
-            } else {
-                PTTA_TRY(conv_fwd(Wt.e1b, A.t1, A.x1, PRO_NONE, nullptr, 0, A.x1r.p, nullptr, pre_x3->p));
-            }
+        if (pre_x3 && up2_in_epilogue(Wt.e1b, A.t1)) {
+            PTTA_TRY(conv_fwd(Wt.e1b, A.t1, A.x1, PRO_NONE, nullptr, 0, A.x1r.p, nullptr, pre_x3->p));
         } else {
             PTTA_TRY(conv_fwd(Wt.e1b, A.t1, A.x1, PRO_NONE, nullptr, 0, pre_x3 ? nullptr : A.x1r.p));
             if (pre_x3) PTTA_TRY(add_up2(A.x1, *pre_x3, A.x1r.p));
         }
         PTTA_TRY(conv_fwd(Wt.e2a, A.x1r, A.t2, PRO_NONE, nullptr, 1));
-        if (pre_x2 && can_fuse_up2(Wt.e2b, A.t2)) {
+        if (pre_x2 && up2_in_epilogue(Wt.e2b, A.t2)) {
             PTTA_TRY(conv_fwd(Wt.e2b, A.t2, A.x2, PRO_NONE, nullptr, 0, nullptr, nullptr, pre_x2->p));
         } else {
             PTTA_TRY(conv_fwd(Wt.e2b, A.t2, A.x2, PRO_NONE));
@@ -1015,25 +974,17 @@ struct ptta_msgchn {
         {   // x2 = dx2 + cx2 (and ReLU(x2)), x1 = dx1 + cx1, x0 = dx0 + cx0 in one launch
             DecSumsParams dp;
             dp.a[0] = E.x2.p; dp.b[0] = cx2.p; dp.out[0] = A.x2.p; dp.n8[0] = (long long)A.x2.numel() / 8;
-            dp.a[1] = E.x1.p; dp.b[1] = cx1.p; dp.out[1] = A.x1.p; dp.n8[1] = E.sum1_done ? 0 : (long long)A.x1.numel() / 8;
-            dp.a[2] = E.x0.p; dp.b[2] = cx0.p; dp.out[2] = A.x0.p; dp.n8[2] = E.sum0_done ? 0 : (long long)A.x0.numel() / 8;
+            dp.a[1] = E.x1.p; dp.b[1] = cx1.p; dp.out[1] = A.x1.p; dp.n8[1] = (long long)A.x1.numel() / 8;
+            dp.a[2] = E.x0.p; dp.b[2] = cx0.p; dp.out[2] = A.x0.p; dp.n8[2] = (long long)A.x0.numel() / 8;
             dp.out0_relu = A.x2r.p;
             launch_k(dec_sums_kernel, cdiv(dp.n8[0] + dp.n8[1] + dp.n8[2], 256), 256, 0, st, dp);
             PTTA_TRY(check_launch("dec_sums"));
         }
         // x2r, u2, s1, u1, s0, h hold ReLU(.): each is read through a ReLU only (forward) or as a ReLU mask (backward)
         PTTA_TRY(conv_fwd(Wt.d2a, A.x2r, A.u2, PRO_NONE, nullptr, 1));
-        if (fuse_dec_sums) {
-            PTTA_TRY(conv_fwd(Wt.d2b, A.u2, A.x3, PRO_NONE, nullptr, 0, A.s1.p, A.x1.p));      // x3, and s1 = ReLU(x1 + x3) from the same epilogue
-            PTTA_TRY(conv_fwd(Wt.d1a, A.s1, A.u1, PRO_NONE, nullptr, 1));
-            PTTA_TRY(conv_fwd(Wt.d1b, A.u1, A.x4, PRO_NONE, nullptr, 0, A.s0.p, A.x0.p));      // x4, and s0 = ReLU(x4 + x0)
-        } else {
-            PTTA_TRY(conv_fwd(Wt.d2b, A.u2, A.x3, PRO_NONE));
-            PTTA_TRY(add32(A.x1, A.x3, A.s1, 1));
-            PTTA_TRY(conv_fwd(Wt.d1a, A.s1, A.u1, PRO_NONE, nullptr, 1));
-            PTTA_TRY(conv_fwd(Wt.d1b, A.u1, A.x4, PRO_NONE));
-            PTTA_TRY(add32(A.x4, A.x0, A.s0, 1));
-        }
+        PTTA_TRY(conv_fwd(Wt.d2b, A.u2, A.x3, PRO_NONE, nullptr, 0, A.s1.p, A.x1.p));      // x3, and s1 = ReLU(x1 + x3) from the same epilogue
+        PTTA_TRY(conv_fwd(Wt.d1a, A.s1, A.u1, PRO_NONE, nullptr, 1));
+        PTTA_TRY(conv_fwd(Wt.d1b, A.u1, A.x4, PRO_NONE, nullptr, 0, A.s0.p, A.x0.p));      // x4, and s0 = ReLU(x4 + x0)
         PTTA_TRY(conv_fwd(Wt.p1, A.s0, A.h, PRO_NONE, nullptr, 1));
         return head_fwd(Wt.p3, A.h, add, out);
     }
@@ -1041,11 +992,10 @@ struct ptta_msgchn {
         if (is_real && !enc1_done) PTTA_TRY(run_encoder(enc1W, B.e1, d14.p, nullptr, nullptr, nullptr, nullptr));
         PTTA_TRY(run_decoder(dec1W, B.d1, B.e1, B.c[2], B.c[3], B.c[4], nullptr, B.d1.out));
         PTTA_TRY(up2_1(B.d1.out, nullptr, nullptr, B.p12));                        // p12 = up2(out14)
-        PTTA_TRY(run_encoder(enc2W, B.e2, d12.p, B.p12.p, &B.d1.x4, &B.d1.x3, &B.d1.x2, &B.d2.x0, &B.c[1], &B.d2.x1, &B.c[2]));
+        PTTA_TRY(run_encoder(enc2W, B.e2, d12.p, B.p12.p, &B.d1.x4, &B.d1.x3, &B.d1.x2));
         PTTA_TRY(run_decoder(dec2W, B.d2, B.e2, B.c[1], B.c[2], B.c[3], nullptr, B.d2.out));
         PTTA_TRY(up2_1(B.d2.out, B.p12.p, nullptr, B.p11));                        // p11 = up2(out12 + p12)
-        if (is_real) PTTA_TRY(run_encoder(enc3W, B.e3, dcl.p, B.p11.p, &B.d2.x4, &B.d2.x3, &B.d2.x2, &B.d3.x0, &B.c[0], &B.d3.x1, &B.c[1]));
-        else PTTA_TRY(run_encoder(enc3W, B.e3, dcl.p, B.p11.p, &B.d2.x4, &B.d2.x3, &B.d2.x2));      // no decoder 3 on the zero-image branch
+        PTTA_TRY(run_encoder(enc3W, B.e3, dcl.p, B.p11.p, &B.d2.x4, &B.d2.x3, &B.d2.x2));
         if (!is_real) return 0;                                                    // zero branch stops after encoder 3
         if (mlp_on_st3) {
             // ref = proj(z_real) needs e3.x2 only: it runs on the second side stream while decoder 3 runs here
@@ -2166,10 +2116,6 @@ int ptta_msgchn_create(ptta_msgchn** out, int n, int h, int w, const char* prepa
     e->N = e->padded ? 2 * n : n; e->H = (h + 15) / 16 * 16; e->W = (w + 15) / 16 * 16;
     e->two_layers = two; e->prepare_mode = mode;
     e->has_heads = mode.find("selfsup") != std::string::npos;
-    if (getenv("PTTA_NO_TC")) e->tc_enabled = false;
-    if (getenv("PTTA_NO_FUSE_DEC_SUMS")) e->fuse_dec_sums = false;
-    if (getenv("PTTA_ONE_STREAM")) e->two_streams = false;
-    if (const char* v = getenv("PTTA_TC_MIN_PIXELS")) e->tc_min_pixels = e->tc_s2_min_pixels = e->tc_t2_min_pixels = e->tc_head_min_pixels = e->tc_stem_min_pixels = atoll(v);
     e->define_model();
     e->plan();
     *out = e;
@@ -2257,11 +2203,7 @@ int ptta_msgchn_set_option(ptta_msgchn* e, const char* name, long long value) {
     else if (k == "tc_stem_min_pixels") e->tc_stem_min_pixels = value;  // same for the {1,2,3} -> 32 tcgen05 stem (and the prediction layers' data gradient)
     else if (k == "tc_enabled") e->tc_enabled = value != 0;
     else if (k == "two_streams") e->two_streams = value != 0;
-    else if (k == "fuse_dec_sums") e->fuse_dec_sums = value != 0;
     else if (k == "fuse_projpred") e->fuse_projpred = value != 0;
-    else if (k == "fuse_up2") e->fuse_up2 = value != 0;
-    else if (k == "fuse_bn_finalize") e->fuse_bn_finalize = value != 0;
-    else if (k == "fuse_enc_sums") e->fuse_enc_sums = value != 0;
     else if (k == "trainable_head") { if (value) PTTA_TRY(e->select_trainable_head()); }   // stage-2 trainer: Adam steps pred.*, not the meta layer
     else if (k == "skip_dec3") e->skip_dec3 = value != 0;                  // stage 2 never reads the prediction of the real branch
     else PTTA_CHECK(false, "set_option: unknown option '%s'", name);

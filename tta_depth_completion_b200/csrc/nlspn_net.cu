@@ -85,16 +85,8 @@ int ptta_nl_stem(const float* image, const float* depth, const float* w_rgb, con
                  const float* scale, const float* shift, void* out, int n, int h, int w, ptta_stream_t stream) {
     PTTA_CHECK(depth && w_rgb && b_rgb && w_dep && b_dep && out, "nl_stem: null pointer");
     const long long total = (long long)n * h * w;
-    launch_k(nl_stem_kernel, cdiv(total, 128), 128, 0, (cudaStream_t)stream, image, depth, w_rgb, b_rgb, w_dep, b_dep, scale, shift, (bf16*)out, n, h, w, n);
+    launch_k(nl_stem_kernel, cdiv(total, 128), 128, 0, (cudaStream_t)stream, image, depth, w_rgb, b_rgb, w_dep, b_dep, scale, shift, (bf16*)out, n, h, w);
     return check_launch("nl_stem");
-}
-
-int ptta_nl_stem_pair(const float* image, const float* depth, const float* w_rgb, const float* b_rgb, const float* w_dep, const float* b_dep,
-                      const float* scale, const float* shift, void* out, int n, int h, int w, ptta_stream_t stream) {
-    PTTA_CHECK(image && depth && w_rgb && b_rgb && w_dep && b_dep && out, "nl_stem_pair: null pointer");
-    const long long total = 2LL * n * h * w;
-    launch_k(nl_stem_kernel, cdiv(total, 128), 128, 0, (cudaStream_t)stream, image, depth, w_rgb, b_rgb, w_dep, b_dep, scale, shift, (bf16*)out, 2 * n, h, w, n);
-    return check_launch("nl_stem_pair");
 }
 
 int ptta_nl_reduce_blocks(long long rows, int c) {
@@ -118,20 +110,6 @@ int ptta_nl_bn_stats(const void* x, long long ldx, long long rows, int c, const 
     return check_launch("nl_bn_finalize");
 }
 
-int ptta_nl_bn_stats_grouped(const void* x, long long ldx, long long rows_per_group, int groups, int c, const float* gamma, const float* beta,
-                             float eps, float* partial, float* mean, float* rstd, float* scale, float* shift, ptta_stream_t stream) {
-    PTTA_CHECK(x && gamma && beta && partial && mean && rstd && scale && shift && c % 64 == 0 && rows_per_group > 0 && groups >= 1 && groups <= 8,
-               "nl_bn_stats_grouped: bad arguments");
-    const int nblk = ptta_nl_reduce_blocks(rows_per_group, c);
-    dim3 grid(nblk, c / 64, groups);
-    launch_k(chan_reduce_kernel<0>, grid, 256, 0, (cudaStream_t)stream, (const bf16*)x, ldx, nullptr, 0, nullptr, 0, nullptr, 0, nullptr, nullptr, rows_per_group,
-                                                                 c, partial);
-    PTTA_TRY(check_launch("nl_chan_stats_grouped"));
-    launch_k(bn_finalize2_kernel, dim3(cdiv(c, 32), groups), 1024, 0, (cudaStream_t)stream, partial, nblk, rows_per_group, c, gamma, beta, eps, mean, rstd, scale,
-                                                                                    shift, nullptr, nullptr, nullptr, 0.f, nullptr);
-    return check_launch("nl_bn_finalize_grouped");
-}
-
 int ptta_nl_col_sums(const void* x, long long ldx, long long rows, int c, float* partial, float* sums, ptta_stream_t stream) {
     PTTA_CHECK(x && partial && sums && c % 64 == 0 && rows > 0, "nl_col_sums: bad arguments");
     const int nblk = ptta_nl_reduce_blocks(rows, c);
@@ -143,26 +121,12 @@ int ptta_nl_col_sums(const void* x, long long ldx, long long rows, int c, float*
     return check_launch("nl_col_sums");
 }
 
-static int bn_act_launch(const void* x, const float* scale, const float* shift, const void* res, long long ldr, const float* rscale,
-                         const float* rshift, void* y, long long rows, int c, int act, long long rows_per_group, ptta_stream_t stream);
-
 int ptta_nl_bn_act(const void* x, const float* scale, const float* shift, const void* res, long long ldr, const float* rscale,
                    const float* rshift, void* y, long long rows, int c, int act, ptta_stream_t stream) {
-    return bn_act_launch(x, scale, shift, res, ldr, rscale, rshift, y, rows, c, act, 0, stream);
-}
-
-int ptta_nl_bn_act_grouped(const void* x, const float* scale, const float* shift, const void* res, long long ldr, const float* rscale,
-                           const float* rshift, void* y, long long rows_per_group, int groups, int c, int act, ptta_stream_t stream) {
-    PTTA_CHECK(groups >= 1 && rows_per_group > 0, "nl_bn_act_grouped: bad arguments");
-    return bn_act_launch(x, scale, shift, res, ldr, rscale, rshift, y, rows_per_group * groups, c, act, rows_per_group, stream);
-}
-
-static int bn_act_launch(const void* x, const float* scale, const float* shift, const void* res, long long ldr, const float* rscale,
-                         const float* rshift, void* y, long long rows, int c, int act, long long rows_per_group, ptta_stream_t stream) {
     PTTA_CHECK(x && scale && shift && y && c % 64 == 0 && rows > 0 && (!rscale || (res && rshift)), "nl_bn_act: bad arguments");
     const long long total = (rows * (c / 8) + 1) / 2;
     launch_k(bn_act_kernel, cdiv(total, 256), 256, 0, (cudaStream_t)stream, (const bf16*)x, scale, shift, (const bf16*)res, ldr, rscale, rshift, (bf16*)y,
-                                                                     rows, c, act, rows_per_group);
+                                                                     rows, c, act);
     return check_launch("nl_bn_act");
 }
 

@@ -47,7 +47,7 @@ __global__ void __launch_bounds__(128) nl_stem_kernel(const float* __restrict__ 
                                                       const float* __restrict__ w_rgb, const float* __restrict__ b_rgb,
                                                       const float* __restrict__ w_dep, const float* __restrict__ b_dep,
                                                       const float* __restrict__ scale, const float* __restrict__ shift,
-                                                      bf16* __restrict__ out, int N, int H, int W, int n_src) {
+                                                      bf16* __restrict__ out, int N, int H, int W) {
     PDL_SYNC();
     __shared__ float s_w[27 * 48 + 9 * 16];      // [ci*9+tap][48] then [tap][16]
     __shared__ float s_b[64];
@@ -62,10 +62,7 @@ __global__ void __launch_bounds__(128) nl_stem_kernel(const float* __restrict__ 
     const long long HW = (long long)H * W, total = (long long)N * HW;
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= total) return;
-    const int x = idx % W, y = (idx / W) % H, n_out = idx / HW;
-    // pair mode (n_src < N): output images n_src .. N-1 are the zero-image copies of images 0 .. n_src-1 (same sparse depth)
-    const int n = n_out % n_src;
-    const bool has_image = image != nullptr && n_out < n_src;
+    const int x = idx % W, y = (idx / W) % H, n = idx / HW;
     float acc[64];
 #pragma unroll
     for (int c = 0; c < 64; ++c) acc[c] = s_b[c];
@@ -79,7 +76,7 @@ __global__ void __launch_bounds__(128) nl_stem_kernel(const float* __restrict__ 
             if (gx < 0 || gx >= W) continue;
             const long long o = (long long)gy * W + gx;
             const int tap = ky * 3 + kx;
-            if (has_image) {
+            if (image) {
 #pragma unroll
                 for (int ci = 0; ci < 3; ++ci) {
                     const float v = fmaf(__ldg(image + ((long long)n * 3 + ci) * HW + o), nsc[ci], nsh[ci]);
@@ -113,9 +110,6 @@ __global__ void __launch_bounds__(256) chan_reduce_kernel(const bf16* __restrict
                                                           const float* __restrict__ mean, const float* __restrict__ rstd, long long P, int C,
                                                           float* __restrict__ partial) {
     PDL_SYNC();
-    // blockIdx.z = statistics group (independent row ranges of P rows each, e.g. the real / zero-image halves of a merged batch)
-    x += (long long)blockIdx.z * P * ldx;
-    partial += (size_t)blockIdx.z * gridDim.x * 2 * C;
     __shared__ float sh[2][8][64];
     const int cg = threadIdx.x & 7, pl = threadIdx.x >> 3, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int c0 = blockIdx.y * 64 + cg * 8;
@@ -245,9 +239,6 @@ __global__ void __launch_bounds__(1024) bn_finalize2_kernel(const float* __restr
     PDL_SYNC();
     int c;
     double s, q;
-    partial += (size_t)blockIdx.y * nblk * 2 * C;                     // statistics group
-    const int go = blockIdx.y * C;
-    mean += go; rstd += go; scale += go; shift += go;
     if (!partial_sums(partial, nblk, C, c, s, q)) return;
     if (sums_out) { sums_out[c] = (float)s; return; }          // plain column sums (bias gradients)
     bn_finalize2_channel(c, s, q, count, gamma, beta, eps, mean, rstd, scale, shift, run_mean, run_var, nbt, momentum);
@@ -255,7 +246,7 @@ __global__ void __launch_bounds__(1024) bn_finalize2_kernel(const float* __restr
 
 // shared-model mode (SyncBatchNorm): the same statistics over the batches of ALL ranks -- the rank's (sum x, sum x^2) per channel are
 // exchanged through peer memory (peer_comm.cuh) and added in rank order, count = local rows x world.  Every thread of every block reaches
-// the exchange, so the early exit of the non-owner threads comes after it.  One statistics group (gridDim.y == 1).
+// the exchange, so the early exit of the non-owner threads comes after it.
 __global__ void __launch_bounds__(1024) bn_finalize2_sync_kernel(const float* __restrict__ partial, int nblk, long long count, int C,
                                                                 const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
                                                                 float* __restrict__ mean, float* __restrict__ rstd, float* __restrict__ scale,
@@ -313,10 +304,8 @@ __global__ void __launch_bounds__(1024) bn_bwd_finalize2_sync_kernel(const float
 // ---- elementwise -----------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) bn_act_kernel(const bf16* __restrict__ x, const float* __restrict__ scale, const float* __restrict__ shift,
                                                      const bf16* __restrict__ res, long long ldr, const float* __restrict__ rscale,
-                                                     const float* __restrict__ rshift, bf16* __restrict__ y, long long P, int C, int act,
-                                                     long long rows_per_group) {
+                                                     const float* __restrict__ rshift, bf16* __restrict__ y, long long P, int C, int act) {
     PDL_SYNC();
-    // rows_per_group > 0: row p uses the scale / shift vectors of group p / rows_per_group (merged real | zero-image batch)
     // two 16-byte elements per thread, `half` apart, loads first (more bytes in flight per thread)
     const int c8n = C >> 3;
     const long long total = P * c8n, half = (total + 1) >> 1;
@@ -337,17 +326,16 @@ __global__ void __launch_bounds__(256) bn_act_kernel(const bf16* __restrict__ x,
     for (int u = 0; u < 2; ++u) {
         if (!ok[u]) continue;
         const int c0 = cc[u];
-        const int gofs = rows_per_group > 0 ? (int)(pp[u] / rows_per_group) * C : 0;
         float v[8], sc[8], sh[8];
         unpack8(rx[u], v);
-        load8f(scale + gofs + c0, sc); load8f(shift + gofs + c0, sh);
+        load8f(scale + c0, sc); load8f(shift + c0, sh);
 #pragma unroll
         for (int j = 0; j < 8; ++j) v[j] = fmaf(v[j], sc[j], sh[j]);
         if (res) {
             float r[8];
             unpack8(rr[u], r);
             if (rscale) {
-                load8f(rscale + gofs + c0, sc); load8f(rshift + gofs + c0, sh);
+                load8f(rscale + c0, sc); load8f(rshift + c0, sh);
 #pragma unroll
                 for (int j = 0; j < 8; ++j) r[j] = fmaf(r[j], sc[j], sh[j]);
             }

@@ -883,8 +883,8 @@ struct BnParams {
     float momentum, eps;
 };
 
-// The per-channel arithmetic of the two finalize steps, written with explicit roundings (no fused multiply-add left to the compiler) so that
-// the stand-alone finalize kernels and the finalize fused into col_stats give bit-identical vectors.
+// The per-channel arithmetic of the two finalize steps, written with explicit roundings (no fused multiply-add left to the compiler), so
+// that the vectors do not depend on the compiler's contraction choices.
 __device__ __forceinline__ void bn_forward_channel(const BnParams& p, int ch, double a, double b, long long count) {
     const double cnt = (double)count;
     const double m = __ddiv_rn(a, cnt);
@@ -954,25 +954,10 @@ __device__ __forceinline__ bool block_reduce_partials(const double* __restrict__
 }
 
 #define STATS_ROWS_PER_BLOCK 64
-// Fused finalize (single-GPU path): instead of a separate bn_finalize / bn_bwd_finalize launch, the LAST blocks of col_stats to finish
-// turn the partial sums into the per-channel vectors.  Every block takes a ticket when its partials are written; the blocks holding the
-// last G tickets (G = number of 32-channel groups, at most the grid size) wait until all tickets are out -- every other block has then
-// published its partials -- and each finalises one group: the same slices, the same summation order and the same arithmetic as the
-// stand-alone finalize kernels, so the vectors are bit-identical to theirs.  At most G blocks ever wait and every block they wait for is
-// already running or does not need their slot, so the wait cannot deadlock.  The last finaliser resets the two counters.
-struct StatsFin {
-    int kind;                     // 0: none, 1: forward (BnParams), 2: backward (dgamma / dbeta / k0 / k1 / k2)
-    unsigned int* counters;       // [2]: tickets, finished finalisers (zero between launches)
-    long long count;
-    BnParams p;
-    const float* gamma; const float* invstd; float* dgamma; float* dbeta; float* k0; float* k1; float* k2;
-};
-__device__ __forceinline__ void stats_fused_finalize(const StatsFin& fin, const double* __restrict__ partial, int nblk, int C, double* scratch);
-
 __global__ void __launch_bounds__(256) col_stats_kernel(const bf16* __restrict__ x, const bf16* __restrict__ dy, double* __restrict__ partial,
                                                         long long rows, int C, int mode, const float* __restrict__ mean,
                                                         const float* __restrict__ invstd, const float* __restrict__ scale,
-                                                        const float* __restrict__ shift, int relu_mask, const StatsFin fin) {
+                                                        const float* __restrict__ shift, int relu_mask) {
     PDL_SYNC();
     extern __shared__ double s_red[];   // [256][2]... reduced per chunk below
     const int CH = C / 8;
@@ -1033,81 +1018,6 @@ __global__ void __launch_bounds__(256) col_stats_kernel(const bf16* __restrict__
         for (int k = 0; k < step; ++k) { a += sh0[(size_t)k * C + ch]; b += sh1[(size_t)k * C + ch]; }
         partial[((size_t)blockIdx.x * 2 + 0) * C + ch] = a;
         partial[((size_t)blockIdx.x * 2 + 1) * C + ch] = b;
-    }
-    if (fin.kind) stats_fused_finalize(fin, partial, (int)gridDim.x, C, s_red);      // s_red (32 KB) is free again: reused for the slice sums
-}
-
-
-// one 32-channel group finalised by a 256-thread block: thread (cx = tid & 31, w = tid >> 5) computes slices ks = w, w + 8, w + 16, w + 24 of
-// the FIN_SLICES = 32 slice sums exactly as block_reduce_partials does with 1024 threads (same loop, same 4-way split, same pairing), then
-// the owner thread adds the 32 slices in the same order
-__device__ __forceinline__ bool group_reduce_partials_256(const double* __restrict__ partial, int nblk, int C, int group, int& ch, double& a, double& b,
-                                                          double (*sh)[FIN_SLICES][32]) {
-    const int cx = threadIdx.x & 31, w = threadIdx.x >> 5;
-    ch = group * 32 + cx;
-    for (int ks = w; ks < FIN_SLICES; ks += 8) {
-        double sa = 0.0, sb = 0.0;
-        if (ch < C) {
-            double a4[4] = {0.0, 0.0, 0.0, 0.0}, b4[4] = {0.0, 0.0, 0.0, 0.0};
-            int k = ks;
-            for (; k + 3 * FIN_SLICES < nblk; k += 4 * FIN_SLICES) {
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    a4[u] += partial[((size_t)(k + u * FIN_SLICES) * 2 + 0) * C + ch];
-                    b4[u] += partial[((size_t)(k + u * FIN_SLICES) * 2 + 1) * C + ch];
-                }
-            }
-            for (; k < nblk; k += FIN_SLICES) {
-                a4[0] += partial[((size_t)k * 2 + 0) * C + ch];
-                b4[0] += partial[((size_t)k * 2 + 1) * C + ch];
-            }
-            sa = (a4[0] + a4[1]) + (a4[2] + a4[3]);
-            sb = (b4[0] + b4[1]) + (b4[2] + b4[3]);
-        }
-        sh[0][ks][cx] = sa; sh[1][ks][cx] = sb;
-    }
-    __syncthreads();
-    a = sh[0][0][cx]; b = sh[1][0][cx];
-    const bool owner = w == 0 && ch < C;
-    if (owner) {
-#pragma unroll
-        for (int k = 1; k < FIN_SLICES; ++k) { a += sh[0][k][cx]; b += sh[1][k][cx]; }
-    }
-    __syncthreads();            // the shared slices are reused by the block's next group
-    return owner;
-}
-
-__device__ __forceinline__ void stats_fused_finalize(const StatsFin& fin, const double* __restrict__ partial, int nblk, int C, double* scratch) {
-    double (*fsh)[FIN_SLICES][32] = reinterpret_cast<double (*)[FIN_SLICES][32]>(scratch);      // 2 x 32 x 32 doubles = 16 KB
-    __shared__ unsigned int s_ticket;
-    __threadfence();                                   // this block's partials are visible device-wide before its ticket is
-    __syncthreads();
-    if (threadIdx.x == 0) s_ticket = atomicAdd(fin.counters, 1u);
-    __syncthreads();
-    const int G = (C + 31) / 32, F = G < nblk ? G : nblk;          // F finaliser blocks: the holders of the last F tickets
-    const int first = nblk - F;
-    if ((int)s_ticket < first) return;
-    if (threadIdx.x == 0) {
-        while (*reinterpret_cast<volatile unsigned int*>(fin.counters) < (unsigned int)nblk) { }
-        __threadfence();
-    }
-    __syncthreads();
-    for (int g = (int)s_ticket - first; g < G; g += F) {
-        int ch; double a, b;
-        const bool owner = group_reduce_partials_256(partial, nblk, C, g, ch, a, b, fsh);
-        if (!owner) continue;
-        if (fin.kind == 1) {
-            bn_forward_channel(fin.p, ch, a, b, fin.count);
-        } else {
-            if (fin.dbeta) fin.dbeta[ch] = (float)a;
-            if (fin.dgamma) fin.dgamma[ch] = (float)b;
-            bn_backward_channel(ch, a, b, fin.count, fin.gamma, fin.invstd, fin.k0, fin.k1, fin.k2);
-        }
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        if (atomicAdd(fin.counters + 1, 1u) == (unsigned int)(F - 1)) { fin.counters[0] = 0u; fin.counters[1] = 0u; __threadfence(); }
     }
 }
 

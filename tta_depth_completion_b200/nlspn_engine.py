@@ -73,10 +73,6 @@ class NlspnEngine:
         self.partial_z = torch.empty_like(self.partial)      # reduction scratch of the zero-image branch (runs on its own stream)
         self.side_stream = torch.cuda.Stream(self.dev)
         self.two_streams = True
-        # option: real + zero-image encoder passes as ONE batch-2N pass (per-half BatchNorm statistics; half the launches, twice the
-        # tiles per conv launch).  Measured at 1x352x1216: 8.86 ms/step against 8.54 ms for the two-stream form, which also overlaps the
-        # zero-image branch with the decoder and the propagation -- so it is off by default
-        self.merge_branches = False
         self.coef = torch.empty(3 * 1024, dtype=torch.float32, device=self.dev)
         self.scratch_c = torch.empty(1024, dtype=torch.float32, device=self.dev)
         self.R = n * (h // 16) * (w // 16)
@@ -107,8 +103,6 @@ class NlspnEngine:
         runs the rendezvous, the epoch advance and the slot parities on a single GPU."""
         self._exchange_at_world1 = bool(exchange_at_world1)
         if comm is not None and (comm.world > 1 or self._exchange_at_world1):
-            if self.merge_branches:
-                raise NotImplementedError('NLSPN shared-model mode: merge_branches (batch-2N encoder) has no SyncBatchNorm form')
             if comm.grad_floats < self.flat_g.numel():
                 raise RuntimeError('NLSPN shared-model mode: the communicator holds %d gradient floats, the model has %d'
                                    % (comm.grad_floats, self.flat_g.numel()))
@@ -357,61 +351,6 @@ class NlspnEngine:
         fe.append(fe6)
         return fe
 
-    # ---- merged real | zero-image encoder -------------------------------------------------------------------------------------------
-    def _bn_layer_grouped(self, key, raw, act, res=None, res_st=None):
-        """train-mode BatchNorm of a merged batch: statistics per half (each half is its own forward pass in the reference)"""
-        c = raw.shape[-1]
-        rows_g = raw.numel() // c // 2
-        st = self.bn_state.get('m.' + key)
-        if st is None:
-            st = {k: torch.empty(2 * c, dtype=torch.float32, device=self.dev) for k in ('mean', 'rstd', 'scale', 'shift')}
-            self.bn_state['m.' + key] = st
-            self.bn_state['r.' + key] = {k: v[:c] for k, v in st.items()}          # what the backward of the real half reads
-        check(_lib.lib().ptta_nl_bn_stats_grouped(ptr(raw), c, rows_g, 2, c, ptr(self.sd[key + '.weight']), ptr(self.sd[key + '.bias']), BN_EPS,
-                                                  ptr(self.partial), ptr(st['mean']), ptr(st['rstd']), ptr(st['scale']), ptr(st['shift']), _stream()),
-              'nl_bn_stats_grouped')
-        self.launches += 2
-        if act is None:
-            return None, st
-        y = self.buf('m.' + key + '.act', raw.shape)
-        check(_lib.lib().ptta_nl_bn_act_grouped(ptr(raw), ptr(st['scale']), ptr(st['shift']), ptr(res), c, ptr(res_st['scale']) if res_st else None,
-                                                ptr(res_st['shift']) if res_st else None, ptr(y), rows_g, 2, c, act, _stream()), 'nl_bn_act_grouped')
-        self.launches += 1
-        return y, st
-
-    def encoder_merged(self, image, depth):
-        """both encoder passes of nlspnmodel_adapt.py:866-880 / 905-914 as one batch of 2N images (real first, zero-image second)"""
-        sd, N, H, W = self.sd, self.N, self.H, self.W
-        x1 = self.buf('m.stem', (2 * N, H, W, 64))
-        check(_lib.lib().ptta_nl_stem_pair(ptr(image), ptr(depth), ptr(sd['conv1_rgb.0.weight']), ptr(sd['conv1_rgb.0.bias']),
-                                           ptr(sd['conv1_dep.0.weight']), ptr(sd['conv1_dep.0.bias']), ptr(self.img_scale), ptr(self.img_shift), ptr(x1),
-                                           N, H, W, _stream()), 'nl_stem_pair')
-        self.launches += 1
-        x = self.conv('meta', x1, out_name='m.fe1')
-        fe = [x]
-        for name, cin, cout, blocks, stride in RESNET34_LAYERS:
-            for b in range(blocks):
-                p = '%s.%d' % (name, b)
-                c1 = self.conv(p + '.conv1', x, out_name='m.' + p + '.c1')
-                a1, _ = self._bn_layer_grouped(p + '.bn1', c1, ACT_RELU)
-                c2 = self.conv(p + '.conv2', a1, out_name='m.' + p + '.c2')
-                if (p + '.down') in self.C:
-                    cd = self.conv(p + '.down', x, out_name='m.' + p + '.cd')
-                    _, std = self._bn_layer_grouped(p + '.downsample.1', cd, None)
-                    x, _ = self._bn_layer_grouped(p + '.bn2', c2, ACT_RELU, res=cd, res_st=std)
-                else:
-                    x, _ = self._bn_layer_grouped(p + '.bn2', c2, ACT_RELU, res=x)
-            fe.append(x)
-        c6 = self.conv('conv6', x, out_name='m.conv6.raw')
-        fe6, _ = self._bn_layer_grouped('conv6.1', c6, ACT_LEAKY)
-        fe.append(fe6)
-        # the backward pass and the decoder read the real half under the names of the unmerged path
-        for k in [k for k in self.B if k.startswith('m.')]:
-            self.B['r.' + k[2:]] = self.B[k][:N]
-            self.B['z.' + k[2:]] = self.B[k][N:]
-        return fe
-
-
     def _fused_dec1_params(self):
         w = self.flat_p[self.fused_bn_w:self.fused_bn_w + 192]
         b = self.flat_p[self.fused_bn_b:self.fused_bn_b + 192]
@@ -488,23 +427,6 @@ class NlspnEngine:
         main = torch.cuda.current_stream()
         # shared-model mode: one stream (the exchanging kernels of the two branches must not wait on each other across streams)
         side = self.side_stream if (self.two_streams and not self._syncing) else main
-        if self._syncing and self.merge_branches:
-            raise NotImplementedError('NLSPN shared-model mode: merge_branches (batch-2N encoder) has no SyncBatchNorm form')
-        if self.merge_branches and image is not None:
-            fe_m = self.encoder_merged(image, sparse_depth)
-            fe = [t[:self.N] for t in fe_m]
-            self.fe = fe
-            z_zero = fe_m[-1][self.N:].reshape(self.R, 512)
-            if side is not main:
-                side.wait_stream(main)
-            with torch.cuda.stream(side):                      # the heads of the zero rows run beside the decoder
-                emb = self.mlp('z.', 'pred', self.mlp('z.', 'proj', z_zero))
-            out = self.decoder(fe, sparse_depth)
-            ref = self.mlp('r.', 'proj_t', fe[-1].reshape(self.R, 512))
-            if side is not main:
-                main.wait_stream(side)
-            self.emb, self.ref = emb, ref
-            return out, emb, ref
         if side is not main:
             side.wait_stream(main)
         with torch.cuda.stream(side):
