@@ -286,6 +286,20 @@ size_t ptta_eval_metrics_workspace_bytes(void);
 int ptta_eval_metrics(const float* output_depth, const float* ground_truth, long long n, float min_depth, float max_depth,
                       void* workspace, float* result5, ptta_stream_t stream);
 
+/* eval-time hole filling of the NLSPN prediction (src/nlspn_model_adapt.py:124-127 -> src/data_utils.py:327-354): every pixel of
+ * depth [n,1,h,w] (fp32) that is exactly 0 is replaced by skimage.restoration.inpaint_biharmonic of its sample, solved exactly in fp64
+ * (block Cholesky per connected component of the holes, csrc/inpaint.cuh) and clipped to the range of the sample's known pixels.
+ * ptta_inpaint_plan: summary (device, 4 * n + 4 uint32) = per sample {holes, ~key(min known), key(max known), 0} followed by the
+ *   solve status word; the caller reads the summary back.  No holes anywhere: nothing else to do.
+ * ptta_inpaint_workspace_bytes: from that HOST copy, the solve workspace; fails for a sample without a known pixel (the reference's
+ *   empty `min` raises there).
+ * ptta_inpaint_solve: in place on depth; summary is the device summary of the same depth.  Status word summary[4 * n] afterwards
+ *   (device): 0 ok, 1 non-positive pivot (that component is left NaN), 2 workspace too small.  n * h * w < 2^31. */
+int ptta_inpaint_plan(const float* depth, int n, int h, int w, unsigned int* summary, ptta_stream_t stream);
+int ptta_inpaint_workspace_bytes(const unsigned int* summary_host, int n, int h, int w, size_t* bytes);
+int ptta_inpaint_solve(float* depth, int n, int h, int w, const unsigned int* summary, void* workspace, size_t workspace_bytes,
+                       ptta_stream_t stream);
+
 /* input stage (SURVEY.md 8f rank 2): src/data_utils.py:134-200 (load_image, load_depth_with_validity_map: depth = png / 256,
  * <= 0 -> 0, validity = depth > 0) + the crop of src/datasets.py:83-170, on decoded 8-bit RGB [n,h0,w0,3] and 16-bit depth [n,h0,w0]
  * payloads -> fp32 image NCHW in [0,255], depth and validity [n,1,h,w]; bit-exact with the numpy code */

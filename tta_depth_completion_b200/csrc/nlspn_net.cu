@@ -5,6 +5,7 @@
 #include "common.cuh"
 #include "conv_gen.cuh"
 #include "nlspn_net.cuh"
+#include "inpaint.cuh"
 #include "../../include/ptta_b200.h"
 
 using namespace ptta;
@@ -266,6 +267,62 @@ int ptta_eval_metrics(const float* output_depth, const float* ground_truth, long
     PTTA_TRY(check_launch("eval_metrics"));
     launch_k(eval_metrics_finalize_kernel, 1, 256, 0, (cudaStream_t)stream, (const double*)workspace, blocks, result5);
     return check_launch("eval_metrics_finalize");
+}
+
+int ptta_inpaint_plan(const float* depth, int n, int h, int w, unsigned int* summary, ptta_stream_t stream) {
+    PTTA_CHECK(depth && summary && n >= 1 && h >= 1 && w >= 1 && (long long)n * h * w < (1LL << 31), "inpaint_plan: bad arguments");
+    cudaStream_t st = (cudaStream_t)stream;
+    PTTA_CUDA(cudaMemsetAsync(summary, 0, (4 * (size_t)n + 4) * sizeof(unsigned int), st));
+    const long long hw = (long long)h * w;
+    const int bx = (int)(cdiv(hw, 2048) < 128 ? cdiv(hw, 2048) : 128);
+    launch_k(inpaint_scan_kernel, dim3(bx, n), 256, 0, st, depth, hw, summary);
+    return check_launch("inpaint_scan");
+}
+
+int ptta_inpaint_workspace_bytes(const unsigned int* summary_host, int n, int h, int w, size_t* bytes) {
+    PTTA_CHECK(summary_host && bytes && n >= 1 && h >= 1 && w >= 1 && (long long)n * h * w < (1LL << 31), "inpaint_workspace_bytes: bad arguments");
+    for (int s = 0; s < n; ++s)
+        PTTA_CHECK(summary_host[4 * s] < (unsigned int)((long long)h * w), "inpaint: sample %d has no known pixel (every depth is 0)", s);
+    *bytes = inpaint_layout(n, h, w, inpaint_arena_doubles(summary_host, n, h, w)).total;
+    return 0;
+}
+
+int ptta_inpaint_solve(float* depth, int n, int h, int w, const unsigned int* summary, void* workspace, size_t workspace_bytes,
+                       ptta_stream_t stream) {
+    PTTA_CHECK(depth && summary && workspace && n >= 1 && h >= 1 && w >= 1 && (long long)n * h * w < (1LL << 31), "inpaint_solve: bad arguments");
+    const InpaintLayout L0 = inpaint_layout(n, h, w, 0);
+    PTTA_CHECK(workspace_bytes >= L0.total, "inpaint_solve: workspace of %zu bytes, at least %zu needed", workspace_bytes, L0.total);
+    static const InpaintStencil stencil = inpaint_make_stencil();
+    char* ws = (char*)workspace;
+    cudaStream_t st = (cudaStream_t)stream;
+    const long long total = (long long)n * h * w;
+    InpaintSolveArgs a;
+    a.depth = depth;
+    a.summary = summary;
+    a.label = (const int*)(ws + L0.label);
+    a.index = (int*)(ws + L0.index);
+    a.comp = (const int*)(ws + L0.comp);
+    a.counters = (int*)(ws + L0.counters);
+    a.bump = (unsigned long long*)(ws + L0.counters + 16);
+    a.arena_doubles = (workspace_bytes - L0.arena) / 8;
+    a.arena = (double*)(ws + L0.arena);
+    a.status = (int*)(summary + 4 * (size_t)n);
+    a.scratch = (int*)(ws + L0.scratch);
+    a.scratch_ints = L0.scratch_ints;
+    a.h = h; a.w = w; a.sy_max = L0.sy_max; a.sx_max = L0.sx_max; a.s_max = L0.s_max;
+    a.st = stencil;
+    PTTA_CUDA(cudaMemsetAsync(ws + L0.counters, 0, 64, st));
+    const int blocks = (int)(cdiv(total, 256) < 1184 ? cdiv(total, 256) : 1184);
+    launch_k(inpaint_init_kernel, blocks, 256, 0, st, (const float*)depth, total, (int*)a.label);
+    PTTA_TRY(check_launch("inpaint_init"));
+    launch_k(inpaint_union_kernel, blocks, 256, 0, st, (int*)a.label, total, h, w);
+    PTTA_TRY(check_launch("inpaint_union"));
+    launch_k(inpaint_flatten_kernel, blocks, 256, 0, st, (int*)a.label, total, a.index, (int*)a.comp, a.counters);
+    PTTA_TRY(check_launch("inpaint_flatten"));
+    launch_k(inpaint_stats_kernel, blocks, 256, 0, st, a.label, total, h, w, (const int*)a.index, (int*)a.comp);
+    PTTA_TRY(check_launch("inpaint_stats"));
+    launch_k(inpaint_solve_kernel, INPAINT_SOLVE_CTAS, INPAINT_THREADS, 0, st, a);
+    return check_launch("inpaint_solve");
 }
 
 int ptta_input_stage(const void* image_u8_hwc, const void* depth_u16, float* image_nchw, float* depth, float* validity, int n, int h0, int w0,

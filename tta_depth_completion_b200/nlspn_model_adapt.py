@@ -7,14 +7,16 @@ native engine (nlspn_engine.py): same method names, argument meaning and error t
 
 `forward` returns tensors attached to a custom autograd.Function; `loss.backward()` runs the native backward and leaves `.grad` on
 the 88 adapted nn.Parameters (views of the engine's flat buffer), so the driver's own three lines work unchanged.
-Outside the hot path (DESIGN.md): adapt modes other than 'meta_bn', prepare modes other than '...meta...seq...1layer...ema',
-the eval-time CPU hole filling (`inpainting`, src/nlspn_model_adapt.py:124-127, skimage) -- these raise NotImplementedError or
-are skipped as documented.  No CPU / PyTorch fallback."""
+The eval forward fills the prediction's holes (pixels that are exactly 0) as the reference's `inpainting` does
+(src/nlspn_model_adapt.py:124-127 -> src/data_utils.py:327-354, skimage's biharmonic inpainting on the CPU), here with an exact fp64
+solve on the device (ops.inpaint_biharmonic).  Outside the hot path (DESIGN.md): adapt modes other than 'meta_bn', prepare modes other
+than '...meta...seq...1layer...ema' -- these raise NotImplementedError.  No CPU / PyTorch fallback."""
 import math
 from collections import OrderedDict
 
 import torch
 
+from . import ops
 from .nlspn_engine import NlspnEngine, adapt_parameter_names, RESNET34_LAYERS
 
 
@@ -145,7 +147,6 @@ class NLSPNModel_Adapt(object):
         self.legacy = bool(offset)               # src/nlspn_model_adapt.py:62: args.legacy = offset
         self.prop_time = 18
         self.training = True
-        self.warn_on_holes = True               # eval forward: one device->host read to report holes the reference would inpaint (False: skip the check)
         self.prepare_mode = None
         self.adapt = False
         self._sd = None
@@ -215,17 +216,11 @@ class NLSPNModel_Adapt(object):
         eng.repack_adapted()
         with torch.no_grad():
             out = eng.forward(image, sparse_depth, training=False)
-        # the reference fills holes (pixels that are exactly 0) with skimage's inpaint_biharmonic on the CPU here
-        # (src/nlspn_model_adapt.py:124-127 -> src/data_utils.py:327-354) and returns the map untouched when there is none.  The solver is
-        # not reproduced: a prediction without holes is identical to the reference's, one WITH holes is reported instead of passing silently
+        # the reference fills holes (pixels that are exactly 0) with skimage's inpaint_biharmonic here
+        # (src/nlspn_model_adapt.py:124-127 -> src/data_utils.py:327-354) and returns the map untouched when there is none
         out = out.clone()
-        if self.warn_on_holes and 'head' not in loss_type:
-            holes = int((out == 0).sum())
-            if holes:
-                import warnings
-                warnings.warn('NLSPN eval forward: %d of %d predicted depths are exactly 0; the reference would fill them with '
-                              'skimage.restoration.inpaint_biharmonic (src/data_utils.py:327-354), this path returns them as they are'
-                              % (holes, out.numel()), RuntimeWarning)
+        if 'head' not in loss_type:
+            ops.inpaint_biharmonic(out)
         return out
 
     def parameters(self):

@@ -351,6 +351,37 @@ def eval_metrics(output_depth, ground_truth, min_depth, max_depth):
     return {'mae': float(v[0]), 'rmse': float(v[1]), 'imae': float(v[2]), 'irmse': float(v[3]), 'count': int(v[4])}
 
 
+def inpaint_biharmonic(depth):
+    """In place on a contiguous CUDA fp32 [N,1,H,W] map: every pixel that is exactly 0 becomes
+    skimage.restoration.inpaint_biharmonic of its sample, clipped to the range of the sample's known pixels (the reference's eval-time
+    hole filling, src/nlspn_model_adapt.py:124-127 -> src/data_utils.py:327-354), solved exactly in fp64 on the device.  One read of a
+    4 x N word summary; when it shows holes, the solve runs and its status word is read back.  A sample whose pixels are all 0 raises
+    ValueError, as the reference's empty `min` does.  Returns `depth`."""
+    _need(depth, torch.float32, 'depth')
+    if depth.dim() != 4 or depth.shape[1] != 1:
+        raise ValueError('inpaint_biharmonic expects [N,1,H,W], got %s' % (tuple(depth.shape),))
+    n, _, h, w = depth.shape
+    L = _lib.lib()
+    summary = torch.empty(4 * n + 4, dtype=torch.int32, device=depth.device)
+    check(L.ptta_inpaint_plan(ptr(depth), n, h, w, ptr(summary), _stream()), 'inpaint_plan')
+    host = summary.cpu()
+    holes = host[0:4 * n:4]
+    if not bool(holes.any()):
+        return depth
+    full = (holes == h * w).nonzero().flatten().tolist()
+    if full:
+        raise ValueError('zero-size array to reduction operation minimum which has no identity (sample %d of the prediction is 0 everywhere)'
+                         % full[0])
+    nbytes = ctypes.c_size_t()
+    check(L.ptta_inpaint_workspace_bytes(c_void_p(host.data_ptr()), n, h, w, ctypes.byref(nbytes)), 'inpaint_workspace_bytes')
+    ws = torch.empty(nbytes.value, dtype=torch.uint8, device=depth.device)
+    check(L.ptta_inpaint_solve(ptr(depth), n, h, w, ptr(summary), ptr(ws), nbytes.value, _stream()), 'inpaint_solve')
+    status = int(summary[4 * n])
+    if status:
+        raise RuntimeError('inpaint_biharmonic: solve status %d (%s)' % (status, 'non-positive pivot' if status == 1 else 'workspace too small'))
+    return depth
+
+
 def input_stage(image_u8_hwc, depth_u16, crop_shape=None, crop_type=('bottom',), depth_multiplier=256.0):
     """Decoded 8-bit RGB [N,H0,W0,3] (uint8) and 16-bit depth [N,H0,W0] (int16/uint16 bit pattern) -> (image fp32 NCHW in [0,255],
     sparse depth, validity map), cropped like the reference's default crop (src/datasets.py:83-170: horizontally centred, vertically
